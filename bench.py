@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the NIS hot path (BASELINE.json): fused flow forward + log-det, points/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (N=1 and per GPU for N>1, weak scaling): BASELINE.json configs[1] — 8D, PWLinear coupling,
 6 cells, 32 bins, conditioner [64]*3, forward + Jacobian on 2^22 synthetic uniform points per step,
@@ -27,6 +27,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -37,6 +38,8 @@ IO_BYTES_PER_POINT = 68          # fp32 in 32 B + out 36 B
 RAMBO_EVENTS = 1 << 24
 RAMBO_BYTES_PER_EVENT = 264      # fp64: 8 uniforms in + (6x4 momenta + weight) out
 METRIC = "nis_flow_fwd_logdet_points_per_sec"
+DUMP_ROWS = 1 << 20              # --dump-outputs: 2^20 of the 2^22 output rows, 36 MB of float32
+DUMP_SEED = 2027
 
 
 def peaks():
@@ -125,6 +128,16 @@ def time_steps(fn, steps, warmup, world, join=None):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     return float(ms.item()) / steps
+
+
+def dump_outputs(path, XJ):
+    """Writes what one flow step returns to its caller, XJ [N, 9] (the eight mapped coordinates, then the Jacobian),
+    as path/xj.npy (float32), so that two builds can be compared output for output.  The whole output is larger than
+    a comparison needs, so the rows written are a fixed sample: DUMP_ROWS distinct row indices drawn with DUMP_SEED,
+    in increasing order."""
+    rows = torch.randperm(XJ.shape[0], generator=torch.Generator().manual_seed(DUMP_SEED))[:DUMP_ROWS].sort().values
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "xj.npy"), XJ.index_select(0, rows.to(XJ.device)).float().cpu().numpy())
 
 
 def fma_peak_tflops():
@@ -583,7 +596,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip cpu baseline / rambo / eval-mode extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the rows the last step returned to DIR/xj.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -613,6 +630,7 @@ def main():
                    generator=torch.Generator(device=dev).manual_seed(2026 + rank))
     moments = torch.zeros(3, dtype=torch.double, device=dev)
     rws = torch.empty(lib.nis_reduce_workspace_bytes(), dtype=torch.uint8, device=dev)
+    last = {}
 
     def step():
         with torch.no_grad():
@@ -622,6 +640,8 @@ def main():
             lib.nis_reduce_moments(_cabi.ptr(J), _cabi.F32, J.numel(), _cabi.ptr(moments), 0, _cabi.ptr(rws),
                                    rws.numel(), _cabi.stream_ptr(dev))
             dist.all_reduce(moments)
+        if args.dump_outputs:
+            last["XJ"] = XJ
         return XJ
 
     sampler = ClockSampler(local)
@@ -629,6 +649,9 @@ def main():
         sampler.start()
     ms = time_steps(step, args.steps, args.warmup, world)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["XJ"])
+    last.clear()
     value = world * N_POINTS / (ms * 1e-3)
     n_cells, depth = 6, 3
     # counted, not assumed: the library marks every kernel it launches for one forward (two weight packs, the first cell's
@@ -782,15 +805,15 @@ def main():
         model.train()
         del x
         torch.cuda.empty_cache()
-        line["rambo"] = bench_rambo(max(3, args.steps // 2), args.warmup, world, pk["hbm_gbs"], peak_kind)
-        line["train_step"] = bench_train_step(max(3, args.steps // 2), args.warmup, world, dev)
-        line["train_step_large"] = bench_train_step(max(3, args.steps // 2), args.warmup, world, dev, log2n=20)
+        line["rambo"] = bench_rambo(args.steps, args.warmup, world, pk["hbm_gbs"], peak_kind)
+        line["train_step"] = bench_train_step(args.steps, args.warmup, world, dev)
+        line["train_step_large"] = bench_train_step(args.steps, args.warmup, world, dev, log2n=20)
         line["integrate"] = bench_integrate(world, dev)
         par = parity_checks(rank, world, dev)
         par["integrate_finite"] = line["integrate"]["finite"]
         par["integrate_within_one_honest_error"] = line["integrate"]["within_one_honest_error"]
         line["parity"] = par
-        line["wide_flow"] = bench_wide(max(3, args.steps // 2), args.warmup, world, dev)
+        line["wide_flow"] = bench_wide(args.steps, args.warmup, world, dev)
         if world == 1:
             line["readme_example"] = bench_readme(dev)
         if rank == 0 and world == 1:

@@ -43,15 +43,17 @@ def _worker(rank, world, port, out):
         expect[1] = 1.0                                    # rank 1 had no gradient there
         grads_ok = all(torch.allclose(p.grad, torch.full_like(p, e)) for p, e in zip(params, expect))
         # fast path: the gradients are views of ONE flat buffer (what nis_flow_backward + autograd leave behind):
-        # a single in-place collective, the views stay views
-        flat = torch.arange(sum(p.numel() for p in params), dtype=torch.float32) * (rank + 1)
+        # a single in-place collective, the views stay views; the buffer lives where the parameters do (create_model
+        # places them on cuda:0 when a GPU is present)
+        dev = params[0].device
+        flat = torch.arange(sum(p.numel() for p in params), dtype=torch.float32, device=dev) * (rank + 1)
         off = 0
         for p in params:
             p.grad = flat[off:off + p.numel()].view(p.shape)
             off += p.numel()
         ptrs = [p.grad.data_ptr() for p in params]
         BasicManager._allreduce_grads(params)
-        want = torch.arange(flat.numel(), dtype=torch.float32) * (world * (world + 1) / 2)
+        want = torch.arange(flat.numel(), dtype=torch.float32, device=dev) * (world * (world + 1) / 2)
         grads_ok = grads_ok and torch.equal(flat, want) and ptrs == [p.grad.data_ptr() for p in params] and \
             torch.equal(torch.cat([p.grad.reshape(-1) for p in params]), want)
         # latent-point streams: identical user seed on every rank -> different points per rank, same on re-run
