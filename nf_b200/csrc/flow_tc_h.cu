@@ -133,16 +133,18 @@ __global__ void __launch_bounds__(256) flow_h_pack_kernel(DevFlow F, const float
 
 struct HSmem {      // byte offsets from the 1024-aligned base
     int w0, aff, bias, st, sst, red, zb, total;
-    int wl[NIS_MAX_HIDDEN + 1];     // per MMA layer l (1..depth): offset of (hi, lo), or -1 when not staged
+    int wfirst;     // the staged MMA layers wfirst .. l_end (hi, lo) start at offset 0, hidden ones 16 KB apart, the
+                    // output layer (l = depth) last
+    // offset of staged layer l: a closed form, so that the kernel indexes no array (which would live in local memory:
+    // a 136-byte stack frame, reloaded in the tile loop)
+    __host__ __device__ int wl(int l) const { return (l - wfirst) * H_HID_BYTES; }
 };
 __host__ __device__ static inline HSmem h_layout(const DevFlow& F, int P, int l_begin, int l_end, bool zstage, int NG,
                                                  bool layer0 = true, bool stats = true) {
     HSmem s;
     int o = 0;
-    for (int l = 0; l <= F.depth; ++l) {
-        s.wl[l] = -1;
-        if (l >= 1 && l >= l_begin && l <= l_end) { s.wl[l] = o; o += l == F.depth ? h_out_bytes(F) : H_HID_BYTES; }
-    }
+    s.wfirst = l_begin > 1 ? l_begin : 1;
+    for (int l = s.wfirst; l <= l_end; ++l) o += l == F.depth ? h_out_bytes(F) : H_HID_BYTES;
     (void)P;
     s.w0 = o; o += layer0 ? H_HID_BYTES : 0;                  // layer-0 operand (hi, lo): only when the pass starts from the state
     s.aff = o; o += (F.depth + 1) * 2 * TCH * 4;
@@ -217,6 +219,8 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
     constexpr bool stats = (MODE & 1) != 0;
     constexpr bool from_z = (MODE & 2) != 0;
     constexpr bool nextmom = (MODE & 4) != 0;
+    // the state feeds layer 0, the splines and the stores: a statistics pass from stored activations has none of them
+    constexpr bool needs_state = !(from_z && stats);
     constexpr int MOM_N = 4 + 4 * 5 / 2;                                    // sum x_k, sum x_k x_k2 (k <= k2), P <= 4
     float macc[nextmom ? MOM_N : 1];
 #pragma unroll
@@ -232,11 +236,10 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
     const float* inv_scale = reinterpret_cast<const float*>(cellpack + h_cell_bytes(F) - 64);    // [l] = 1 / (SA * SW_l)
 
     // ---- one-time setup: weights, barriers, tensor memory ---------------------------------------------
-    for (int l = lz; l <= l_end; ++l) {
-        if (L.wl[l] < 0) continue;
+    for (int l = L.wfirst; l <= l_end; ++l) {
         const int n16 = (l == depth ? h_out_bytes(F) : H_HID_BYTES) / 16;
         const uint4* src = reinterpret_cast<const uint4*>(cellpack + (size_t)(l - 1) * H_HID_BYTES);
-        uint4* dst = reinterpret_cast<uint4*>(sm + L.wl[l]);
+        uint4* dst = reinterpret_cast<uint4*>(sm + L.wl(l));
         for (int i = tid; i < n16; i += NT) dst[i] = src[i];
     }
     if (!from_z) {                                                // layer 0 (hi, lo): one K = 16 step of a 64x64 block
@@ -295,7 +298,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
         // (the landing zone is free as soon as every thread has moved its row into its state column)
         float* sst = reinterpret_cast<float*>(sm + L.sst) + g * (d + 1) * TCM;
         const uint32_t SBYTES = (uint32_t)((d + 1) * TCM * 4);
-        const bool st_bulk = A.from_state && (reinterpret_cast<uintptr_t>(A.state_in) & 15) == 0 && (SBYTES & 15) == 0;
+        const bool st_bulk = needs_state && A.from_state && (reinterpret_cast<uintptr_t>(A.state_in) & 15) == 0 && (SBYTES & 15) == 0;
         if (st_bulk && gt == 0) {
             const long long t0 = (long long)blockIdx.x * NG + g;
             if ((t0 + 1) * TCM <= A.B) bulk_load(sst, A.state_in + t0 * TCM * rowlen, SBYTES, &s_full[g]);
@@ -314,7 +317,8 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
             const long long pt = tile * TCM + gt;
             const bool valid = pt < A.B;
             // ---- this thread's point --------------------------------------------------------------
-            if (st_bulk && (tile + 1) * TCM <= A.B) {
+            if (!needs_state) {
+            } else if (st_bulk && (tile + 1) * TCM <= A.B) {
                 mbar_wait(&s_full[g], sph);
                 sph ^= 1;
                 for (int i = 0; i <= d; ++i) st[i * TCM] = sst[gt * rowlen + i];
@@ -395,7 +399,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                 if (gt == 0) {                                    // the group's issuer: all 128 operand rows are in place
                     mbar_wait(&a_ready[g], pa);
                     tc_fence_after();
-                    const uint32_t whi = smem_u32(sm + L.wl[l]);
+                    const uint32_t whi = smem_u32(sm + L.wl(l));
                     const uint32_t tb = tmem_base + g * H_COLS;
                     h_issue_block(tb, tb + H_COL_AHI, tb + H_COL_ALO, whi, whi + (l == depth ? out_rows : TCH) * TCH * 2,
                                   l == depth ? idesc_out : idesc);
@@ -469,7 +473,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                     if (gt == 0) {
                         mbar_wait(&a_ready[g], pa);
                         tc_fence_after();
-                        const uint32_t whi = smem_u32(sm + L.wl[depth]) + (uint32_t)(b + 1) * (K_::OUT_N * 128);
+                        const uint32_t whi = smem_u32(sm + L.wl(depth)) + (uint32_t)(b + 1) * (K_::OUT_N * 128);
                         const uint32_t tb = tmem_base + g * H_COLS;
                         h_issue_block(tb, tb + H_COL_AHI, tb + H_COL_ALO, whi, whi + out_rows * TCH * 2, idesc_out);
                         tc_commit(&d_ready[g]);
