@@ -141,7 +141,8 @@ int nis_flow_backward_cached(const NisFlowDesc* desc, const float* params, const
  * column order -> xj_out [B, n_flow+1] with column n_flow = J_in / prod of the densities, so that
  * nis_flow_inverse(nis_flow_forward(x)) == x with Jacobian 1 (away from PWQuad's clamp at 1 - 1e-6).  EVAL: running
  * statistics; TRAIN: batch statistics of what each cell sees on the way back (running statistics are not updated).
- * Shape-generic FP32 kernels; bins_out as in nis_flow_forward. */
+ * Width-64 PWLin / PWQuad flows with 32 bins (the shapes the fp16-split forward serves) run on the tensor-core kernel, every
+ * other shape on the shape-generic FP32 kernels; bins_out as in nis_flow_forward. */
 int nis_flow_inverse(const NisFlowDesc* desc, const float* params, const float* bn_running,
                      const void* yj_in, int32_t in_dtype, int32_t in_cols,
                      void* xj_out, int32_t out_dtype, int32_t* bins_out, int32_t bn_mode,
@@ -228,8 +229,9 @@ int64_t nis_probe_fp32_fma(float* out, int32_t iters, void* stream);
  * gives the MEASURED tensor-pipe peak the tcgen05 flow kernels are quoted against. */
 int64_t nis_probe_tensor(int32_t kind, int32_t n, int32_t iters, void* stream);
 
-/* Measurement aid for bench.py: per-launch device times of nis_flow_forward.  After nis_flow_timing_begin(stream) every
- * kernel launch of the nis_flow_forward calls made by THIS thread is bracketed by CUDA events recorded on the launch
+/* Measurement aid for bench.py: per-launch device times of nis_flow_forward and nis_flow_inverse.  After
+ * nis_flow_timing_begin(stream) every kernel launch of the nis_flow_forward / nis_flow_inverse calls made by THIS thread
+ * is bracketed by CUDA events recorded on the launch
  * stream; nis_flow_timing_end synchronises them and returns the number of launches written to ms[] / tags[] (tags: 0 weight
  * packs, 1 column moments, 10 fused eval cell, 11 layer pass from the state, 13 layer pass from stored activations, 12
  * final pass from stored activations, 2 other), or a negative error. */

@@ -305,11 +305,12 @@ int nis_launch_col_stats(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
 bool nis_moments_supported(const DevFlow& F, int c);
 int nis_launch_col_moments(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
 
-// ---- measurement aid: per-launch device times of nis_flow_forward (bench.py's roofline object) ---------------------------
-// nis_flow_timing_begin() arms a per-thread sink; every kernel launch of the following nis_flow_forward calls is then
-// bracketed by CUDA events recorded on the launch stream; nis_flow_timing_end() synchronises those events and returns the
-// elapsed time and a tag per launch (0 pack, 1 column moments, 10 + mode for the tensor-core cell kernel: 10 fused cell,
-// 11 layer pass from the state, 12 final pass from stored activations, 13 layer pass from stored activations; 2 other).
+// ---- measurement aid: per-launch device times of nis_flow_forward and nis_flow_inverse (bench.py's roofline object) -----
+// nis_flow_timing_begin() arms a per-thread sink; every kernel launch of the following nis_flow_forward / nis_flow_inverse
+// calls is then bracketed by CUDA events recorded on the launch stream; nis_flow_timing_end() synchronises those events and
+// returns the elapsed time and a tag per launch (0 pack, 1 column moments, 10 + mode for the tensor-core cell kernel: 10
+// fused cell, 11 layer pass from the state, 12 final pass from stored activations, 13 layer pass from stored activations;
+// 2 other, including the shape-generic kernel and the inverse's input gather).
 #define NIS_TIMING_MAX 512
 struct TimingSink { bool on; int n; cudaEvent_t ev[NIS_TIMING_MAX + 1]; int tag[NIS_TIMING_MAX]; bool made; };
 static thread_local TimingSink g_timing = {false, 0, {}, {}, false};
@@ -483,7 +484,7 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
     A.saved = saved; A.bins = bins_out;
     A.params = params; A.wpack = ws.wpack; A.bn_running = bn_running; A.bn_saved = bn_saved;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B;
-    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 0; A.zin_layer = 0; A.next_moments = 0;
+    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 0; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
     // per-cell launch sequences: tcgen05 kernel where it applies, else the FP32 register-tiled kernel
     const bool tc = nis_tc_supported(F, B, bn_mode);
     const bool hp = tc && nis_h_supported(F, B, bn_mode);              // fp16-split, four-group kernel (flow_tc_h.cu)
@@ -598,6 +599,7 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
         const bool last = c == F.n_cells - 1;
         A.next_moments = hp && fuse_env && bn_mode == NIS_BN_TRAIN && !last && A.zin != nullptr
                          && nis_moments_supported(F, c + 1) && F.cells[c + 1].P <= 4;
+        A.next_cell = c + 1;
         moments_ready = A.next_moments != 0;
         A.to_out = last;
         A.state_out = saved ? saved + (long long)(c + 1) * rows : (last ? nullptr : ws.state);
@@ -612,10 +614,93 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
 
 // ---------------------------------------------------------------------------------------------------
 // Inverse flow (SURVEY 8 f4): y -> x with the Jacobian column divided by the product of the densities, so that
-// nis_flow_inverse(nis_flow_forward(x)) = x with Jacobian 1.  Shape-generic kernel only (any shape); eval-mode BN uses
-// the running statistics, train-mode BN the batch statistics of the pass-through columns each cell sees on the way back
-// (the same values as in the forward pass of the same batch); running statistics are not updated.
+// nis_flow_inverse(nis_flow_forward(x)) = x with Jacobian 1.  Eval-mode BN uses the running statistics, train-mode BN the
+// batch statistics of the pass-through columns each cell sees on the way back (the same values as in the forward pass of
+// the same batch); running statistics are not updated.  Width-64 PWLin / PWQuad cells with 32 bins run on the fp16-split
+// tensor-core kernel (flow_tc_h.cu, inverse mode bit), every other shape on the shape-generic kernel.
 // ---------------------------------------------------------------------------------------------------
+
+// input rows [B][in_cols] in the flow's output column order -> float32 state rows [B][d+1] in the physical order (out_perm
+// scatters them back; J = 1 when in_cols = d), so that every inverse cell of the tensor-core path starts from the state
+__global__ void __launch_bounds__(256) flow_inverse_gather_kernel(const __grid_constant__ DevFlow F, const void* __restrict__ in,
+                                                                  int in_dtype, int in_cols, long long B, float* __restrict__ state) {
+    const int d = F.d;
+    const long long n = B * (d + 1);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const long long pt = i / (d + 1);
+        const int r = (int)(i - pt * (d + 1));
+        const float v = (r < d || in_cols > d) ? load_io(in, in_dtype, pt * in_cols + r) : 1.f;
+        state[pt * (d + 1) + (r < d ? F.out_perm[r] : d)] = v;
+    }
+}
+
+// The inverse on the fp16-split kernel: the forward's launch sequence with the cells in reverse order.  The statistics and
+// layer passes are the forward's (they read only the pass-through columns); the fused cell and the final pass run the
+// inverse splines; the fused column moments of a final pass are those of cell c - 1.
+static int inverse_h(const DevFlow& F, FwdArgs A, const FlowWorkspace& ws, int bn_mode, cudaStream_t s) {
+    const long long B = A.B;
+    int rc = nis_h_pack(F, A.params, ws.tcpack, s);
+    if (rc) return rc;
+    timing_mark(s, 0);
+    {
+        const long long n = B * (F.d + 1);
+        const long long nb = (n + 255) / 256;
+        flow_inverse_gather_kernel<<<(unsigned)(nb < 4096 ? nb : 4096), 256, 0, s>>>(F, A.in, A.in_dtype, A.in_cols, B, ws.state);
+        NIS_CUDA_CHECK_LAUNCH();
+        timing_mark(s, 2);
+    }
+    const bool train = bn_mode == NIS_BN_TRAIN;
+    static const int skip_env = [] { const char* e = getenv("NIS_SKIP_LAST_STORE"); return e && e[0] == '0' ? 0 : 1; }();
+    static const int fuse_env = [] { const char* e = getenv("NIS_FUSE_MOMENTS"); return e && e[0] == '0' ? 0 : 1; }();
+    const bool skip_last = skip_env && F.depth >= 3 && F.kind == NIS_KIND_PWLIN;
+    float* zb[2] = {ws.bwd, ws.bwd + zbuf_floats(F, B)};
+    A.from_state = 1; A.state_in = ws.state;
+    bool moments_ready = false;
+    for (int c = F.n_cells - 1; c >= 0; --c) {
+        A.c_begin = c; A.c_end = c + 1;
+        A.state_out = nullptr; A.to_out = 0;
+        A.zin = nullptr; A.zout = nullptr; A.zin_layer = 0; A.next_moments = 0;
+        const bool moments = train && nis_moments_supported(F, c);
+        if (train) {
+            int l0 = 0;
+            if (moments) {
+                if (!moments_ready) {
+                    A.stats_layer = 0;
+                    rc = nis_launch_col_moments(F, A, s);
+                    if (rc) return rc;
+                    timing_mark(s, 1);
+                }
+                l0 = 2;
+            }
+            for (int l = l0; l <= F.depth; ++l) {
+                A.stats_layer = l;
+                if (l >= 1) {
+                    A.zin = (l >= 2 && !(moments && l == 2)) ? zb[(l - 1) & 1] : nullptr;
+                    A.zout = (skip_last && moments && l == F.depth) ? nullptr : zb[l & 1];
+                    rc = nis_launch_h(F, A, ws.tcpack, s);
+                } else {
+                    rc = nis_launch_col_stats(F, A, s);
+                }
+                if (rc) return rc;
+                timing_mark(s, l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
+            }
+        }
+        A.stats_layer = -1;
+        A.zin = (train && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
+        A.zout = nullptr;
+        if (skip_last && moments) { A.zin = zb[(F.depth - 1) & 1]; A.zin_layer = F.depth - 1; }
+        A.next_moments = fuse_env && train && c > 0 && A.zin != nullptr && nis_moments_supported(F, c - 1) && F.cells[c - 1].P <= 4;
+        A.next_cell = c - 1;
+        moments_ready = A.next_moments != 0;
+        A.to_out = c == 0;
+        A.state_out = c == 0 ? nullptr : ws.state;
+        rc = nis_launch_h(F, A, ws.tcpack, s);
+        if (rc) return rc;
+        timing_mark(s, 10 + (A.zin ? 2 : 0));
+    }
+    return NIS_OK;
+}
+
 extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, const float* bn_running,
                                 const void* yj_in, int32_t in_dtype, int32_t in_cols,
                                 void* xj_out, int32_t out_dtype, int32_t* bins_out, int32_t bn_mode,
@@ -641,8 +726,10 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
         }
         int bx = (mx + 255) / 256;
         if (bx > 64) bx = 64;
+        timing_mark(s, -1);
         flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, bn_mode);
         NIS_CUDA_CHECK_LAUNCH();
+        timing_mark(s, 0);
     }
     FwdArgs A;
     A.in = yj_in; A.in_dtype = in_dtype; A.in_cols = in_cols;
@@ -650,11 +737,14 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
     A.saved = nullptr; A.bins = bins_out;
     A.params = params; A.wpack = ws.wpack; A.bn_running = nullptr; A.bn_saved = nullptr;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B;
-    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 1; A.zin_layer = 0; A.next_moments = 0;
+    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 1; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
+    if (nis_tc_supported(F, B, bn_mode) && nis_h_supported(F, B, bn_mode)) return inverse_h(F, A, ws, bn_mode, s);
     if (bn_mode == NIS_BN_EVAL) {
         A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 1;
         A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
-        return launch_fwd_any(F, A, s);
+        rc = launch_fwd_any(F, A, s);
+        if (rc == NIS_OK) timing_mark(s, 2);
+        return rc;
     }
     for (int c = F.n_cells - 1; c >= 0; --c) {
         A.c_begin = c; A.c_end = c + 1;
@@ -665,12 +755,14 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
             A.stats_layer = l;
             rc = launch_fwd_any(F, A, s);
             if (rc) return rc;
+            timing_mark(s, 2);
         }
         A.stats_layer = -1;
         A.to_out = c == 0;
         A.state_out = c == 0 ? nullptr : ws.state;
         rc = launch_fwd_any(F, A, s);
         if (rc) return rc;
+        timing_mark(s, 2);
     }
     return NIS_OK;
 }

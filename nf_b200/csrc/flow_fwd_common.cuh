@@ -20,9 +20,11 @@ struct FwdArgs {
     float* scratch_state;                  // cooperative small-batch kernel: fp32 [B][d+1] state between cells when `saved` is null
     int zin_layer;                         // fp16-split kernel: which layer's pre-activations `zin` holds (0: the default,
                                            // stats_layer - 1 for a layer pass, depth for the final pass)
-    int next_moments;                      // fp16-split final pass: also accumulate the column moments of cell c_begin + 1 (its
+    int next_moments;                      // fp16-split final pass: also accumulate the column moments of cell next_cell (its
                                            // BN_0 / BN_1 statistics) from the state this pass writes - no pass of their own
-    int inverse;                           // nis_flow_inverse: cells backwards, inverse splines, J divided (shape-generic kernel only)
+    int next_cell;                         // the cell that runs after c_begin: c_begin + 1, or c_begin - 1 in the inverse
+    int inverse;                           // nis_flow_inverse: cells backwards, inverse splines, J divided (shape-generic
+                                           // kernel; fp16-split fused cell and final pass)
 };
 
 

@@ -198,7 +198,10 @@ __device__ __forceinline__ void h_issue_block(uint32_t tmem_d, uint32_t t_hi, ui
 
 // MODE: bit 0 = statistics (layer) pass, bit 1 = the first operand comes from stored activations, bit 2 (final pass of a
 // train-mode cell) = the column moments of the NEXT cell's pass-through columns are accumulated from the state this pass
-// writes (14 sums for P <= 4) and folded into that cell's BN_0 / BN_1 by the last CTA.  Compile-time, so that
+// writes (14 sums for P <= 4) and folded into that cell's BN_0 / BN_1 by the last CTA, bit 3 (fused cell or final pass)
+// = the inverse cell (nis_flow_inverse): inverse splines, Jacobian divided by the densities, and the last inverse cell
+// (c = 0) stores the physical column order.  Statistics and layer passes have no inverse bit: they read only the
+// pass-through columns, which a cell conditions on in either direction.  Compile-time, so that
 // every instantiation carries only its own path: the all-in-one kernel was 64 KB of SASS and its four groups, each in
 // another phase, missed the instruction cache (ncu: `no_instruction` 0.8 stalled warps per issue).
 template <int NG, int KIND, int MODE>
@@ -219,6 +222,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
     constexpr bool stats = (MODE & 1) != 0;
     constexpr bool from_z = (MODE & 2) != 0;
     constexpr bool nextmom = (MODE & 4) != 0;
+    constexpr bool inverse = (MODE & 8) != 0;
     // the state feeds layer 0, the splines and the stores: a statistics pass from stored activations has none of them
     constexpr bool needs_state = !(from_z && stats);
     constexpr int MOM_N = 4 + 4 * 5 / 2;                                    // sum x_k, sum x_k x_k2 (k <= k2), P <= 4
@@ -495,50 +499,59 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                         float m = -3.0e38f;
 #pragma unroll
                         for (int j = 0; j < 32; ++j) { z[32 * tt + j] = fmaf(z[32 * tt + j], inv_out, bs[j]); m = fmaxf(m, z[32 * tt + j]); }
-                        // S = sum of the 32 exponentials, C = the kb below the bin, ek = the bin's own: a pairwise sum tree, then
-                        // a descent along the bits of kb that keeps the half / quarter / ... holding the bin (53 selects + 36
-                        // adds; the predicated running sums `C += j < kb ? e : 0`, `ek = j == kb ? e : ek` were 128 + 32)
-                        float e[32], s1[16], s2[8], s4[4];
+                        if (inverse) {
+                            float xo, jinv;
+                            int ki;
+                            pwlin32_tree_inv(z + 32 * tt, m, xv, xo, jinv, ki);
+                            st[q.trafo[t] * TCM] = xo;
+                            jfac *= jinv;
+                            if (A.bins && valid) A.bins[((long long)c * A.B + pt) * d + t] = ki;
+                        } else {
+                            // S = sum of the 32 exponentials, C = the kb below the bin, ek = the bin's own: a pairwise sum tree, then
+                            // a descent along the bits of kb that keeps the half / quarter / ... holding the bin (53 selects + 36
+                            // adds; the predicated running sums `C += j < kb ? e : 0`, `ek = j == kb ? e : ek` were 128 + 32)
+                            float e[32], s1[16], s2[8], s4[4];
 #pragma unroll
-                        for (int j = 0; j < 32; ++j) e[j] = ex2_approx(z[32 * tt + j] - m);
+                            for (int j = 0; j < 32; ++j) e[j] = ex2_approx(z[32 * tt + j] - m);
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) s1[j] = e[2 * j] + e[2 * j + 1];
+                            for (int j = 0; j < 16; ++j) s1[j] = e[2 * j] + e[2 * j + 1];
 #pragma unroll
-                        for (int j = 0; j < 8; ++j) s2[j] = s1[2 * j] + s1[2 * j + 1];
+                            for (int j = 0; j < 8; ++j) s2[j] = s1[2 * j] + s1[2 * j + 1];
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) s4[j] = s2[2 * j] + s2[2 * j + 1];
-                        const float s8a = s4[0] + s4[1], s8b = s4[2] + s4[3];
-                        const float S = s8a + s8b;
-                        const bool b4 = kb & 16, b3 = kb & 8, b2 = kb & 4, b1 = kb & 2, b0 = kb & 1;
-                        float C = b4 ? s8a : 0.f;
+                            for (int j = 0; j < 4; ++j) s4[j] = s2[2 * j] + s2[2 * j + 1];
+                            const float s8a = s4[0] + s4[1], s8b = s4[2] + s4[3];
+                            const float S = s8a + s8b;
+                            const bool b4 = kb & 16, b3 = kb & 8, b2 = kb & 4, b1 = kb & 2, b0 = kb & 1;
+                            float C = b4 ? s8a : 0.f;
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) e[j] = b4 ? e[16 + j] : e[j];
+                            for (int j = 0; j < 16; ++j) e[j] = b4 ? e[16 + j] : e[j];
 #pragma unroll
-                        for (int j = 0; j < 8; ++j) s1[j] = b4 ? s1[8 + j] : s1[j];
+                            for (int j = 0; j < 8; ++j) s1[j] = b4 ? s1[8 + j] : s1[j];
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) s2[j] = b4 ? s2[4 + j] : s2[j];
+                            for (int j = 0; j < 4; ++j) s2[j] = b4 ? s2[4 + j] : s2[j];
 #pragma unroll
-                        for (int j = 0; j < 2; ++j) s4[j] = b4 ? s4[2 + j] : s4[j];
-                        C += b3 ? s4[0] : 0.f;
+                            for (int j = 0; j < 2; ++j) s4[j] = b4 ? s4[2 + j] : s4[j];
+                            C += b3 ? s4[0] : 0.f;
 #pragma unroll
-                        for (int j = 0; j < 8; ++j) e[j] = b3 ? e[8 + j] : e[j];
+                            for (int j = 0; j < 8; ++j) e[j] = b3 ? e[8 + j] : e[j];
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) s1[j] = b3 ? s1[4 + j] : s1[j];
+                            for (int j = 0; j < 4; ++j) s1[j] = b3 ? s1[4 + j] : s1[j];
 #pragma unroll
-                        for (int j = 0; j < 2; ++j) s2[j] = b3 ? s2[2 + j] : s2[j];
-                        C += b2 ? s2[0] : 0.f;
+                            for (int j = 0; j < 2; ++j) s2[j] = b3 ? s2[2 + j] : s2[j];
+                            C += b2 ? s2[0] : 0.f;
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) e[j] = b2 ? e[4 + j] : e[j];
+                            for (int j = 0; j < 4; ++j) e[j] = b2 ? e[4 + j] : e[j];
 #pragma unroll
-                        for (int j = 0; j < 2; ++j) s1[j] = b2 ? s1[2 + j] : s1[j];
-                        C += b1 ? s1[0] : 0.f;
-                        const float e0 = b1 ? e[2] : e[0], e1 = b1 ? e[3] : e[1];
-                        C += b0 ? e0 : 0.f;
-                        const float ek = b0 ? e1 : e0;
-                        const float inv = 1.f / S;
-                        st[q.trafo[t] * TCM] = (ek * alpha + C) * inv;
-                        jfac *= ek * inv * 32.f;
-                        if (A.bins && valid) A.bins[((long long)c * A.B + pt) * d + t] = kb;
+                            for (int j = 0; j < 2; ++j) s1[j] = b2 ? s1[2 + j] : s1[j];
+                            C += b1 ? s1[0] : 0.f;
+                            const float e0 = b1 ? e[2] : e[0], e1 = b1 ? e[3] : e[1];
+                            C += b0 ? e0 : 0.f;
+                            const float ek = b0 ? e1 : e0;
+                            const float inv = 1.f / S;
+                            st[q.trafo[t] * TCM] = (ek * alpha + C) * inv;
+                            jfac *= ek * inv * 32.f;
+                            if (A.bins && valid) A.bins[((long long)c * A.B + pt) * d + t] = kb;
+                        }
                     }
                 } else {
                     // PWQuad, 32 bins (coupling_cells.py:159-228): one transformed dimension per block, 65 logits
@@ -548,7 +561,8 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                     for (int j = 0; j < 65; ++j) z[j] = fmaf(z[j], inv_out, bs[j]);
                     float y, f;
                     int kb;
-                    pwquad32_tree<true>(z, xv, y, f, kb);
+                    if (inverse) pwquad32_tree_inv<true>(z, xv, y, f, kb);      // (f = 1 / density)
+                    else pwquad32_tree<true>(z, xv, y, f, kb);
                     st[q.trafo[b] * TCM] = y;
                     jfac *= f;
                     if (A.bins && valid) A.bins[((long long)c * A.B + pt) * d + b] = kb;
@@ -557,7 +571,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
             st[d * TCM] *= jfac;
             if (nextmom && valid) {
                 // per-thread float32 partials, like flow_col_moments_kernel (a thread sees ~B / (SMs * 512) points <= 1)
-                const DevCell& qn = F.cells[c + 1];
+                const DevCell& qn = F.cells[A.next_cell];
                 float x[4];
 #pragma unroll
                 for (int k = 0; k < 4; ++k) x[k] = k < qn.P ? st[qn.feed[k] * TCM] : 0.f;
@@ -576,7 +590,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                     for (int i = 0; i <= d; ++i) so[i] = st[i * TCM];
                 }
                 if (A.to_out) {
-                    for (int i = 0; i < d; ++i) store_io(A.out, A.out_dtype, pt * rowlen + i, st[F.out_perm[i] * TCM]);
+                    for (int i = 0; i < d; ++i) store_io(A.out, A.out_dtype, pt * rowlen + i, st[(inverse ? i : F.out_perm[i]) * TCM]);
                     store_io(A.out, A.out_dtype, pt * rowlen + d, st[d * TCM]);
                 }
             }
@@ -612,7 +626,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
         if (!s_last_m) return;
         __threadfence();
         fold_partials<MOM_N>(A.partials, gridDim.x, totm + MOM_N, totm, tid, NT);
-        moments_finalize<4>(F, A, c + 1, totm, sc0s_m, tid, NT);
+        moments_finalize<4>(F, A, A.next_cell, totm, sc0s_m, tid, NT);
         if (tid == 0) *A.counter = 0u;
         return;
     }
@@ -697,7 +711,11 @@ static int h_launch_mode(const DevFlow& F, const FwdArgs& A, const char* hpack, 
 
 template <int NG, int KIND>
 static int h_launch(const DevFlow& F, const FwdArgs& A, const char* hpack, size_t smem, int sms, cudaStream_t s) {
-    switch ((A.stats_layer >= 1 ? 1 : 0) | (A.zin != nullptr ? 2 : 0)) {
+    const int mode = (A.stats_layer >= 1 ? 1 : 0) | (A.zin != nullptr ? 2 : 0);
+    if (A.inverse && mode == 0) return h_launch_mode<NG, KIND, 8>(F, A, hpack, smem, sms, s);
+    if (A.inverse && mode == 2) return A.next_moments ? h_launch_mode<NG, KIND, 14>(F, A, hpack, smem, sms, s)
+                                                      : h_launch_mode<NG, KIND, 10>(F, A, hpack, smem, sms, s);
+    switch (mode) {
         case 0: return h_launch_mode<NG, KIND, 0>(F, A, hpack, smem, sms, s);
         case 1: return h_launch_mode<NG, KIND, 1>(F, A, hpack, smem, sms, s);
         case 2: return A.next_moments ? h_launch_mode<NG, KIND, 6>(F, A, hpack, smem, sms, s)
