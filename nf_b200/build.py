@@ -6,7 +6,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnisb200.so")
-SOURCES = ["flow_desc.cu", "flow_fwd.cu", "flow_tiled.cu", "flow_tc.cu", "flow_tc_h.cu", "flow_wide.cu", "flow_bwd.cu", "flow_bwd_tc.cu", "flow_bwd_wide.cu", "rambo.cu", "reduce.cu", "probe_tc.cu"]
+SOURCES = ["flow_desc.cu", "flow_fwd.cu", "flow_tiled.cu", "flow_tc_h.cu", "flow_wide.cu", "flow_bwd.cu", "flow_bwd_tc.cu", "flow_bwd_wide.cu", "rambo.cu", "reduce.cu", "probe_tc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

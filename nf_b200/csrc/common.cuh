@@ -98,7 +98,7 @@ int nis_build_dev_flow(const NisFlowDesc* desc, DevFlow* out);
 // workspace carve-up (all offsets 256-byte aligned)
 struct FlowWorkspace {
     float* wpack;        // [pack_total]
-    float* tcpack;       // tensor-core weight pack (hi/lo TF32 splits in UMMA layout), flow_tc.cu
+    float* tcpack;       // tensor-core weight pack (hi/lo splits in UMMA layout): flow_tc_h.cu, flow_wide.cu, flow_bwd_tc.cu
     float* state;        // [B][d+1] scratch state (train mode without `saved`)
     double* partials;    // [max_grid][2][maxW]
     unsigned* counter;   // last-block ticket

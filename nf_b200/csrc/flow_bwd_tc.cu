@@ -4,7 +4,7 @@
 // (coupling_cells.py:107-142, 230-254) is, per cell and in reverse order, a chain of small GEMMs with a
 // batch-wide BatchNorm reduction between every two of them.  The chain is cut at those reductions:
 //
-//   head   : recompute the conditioner (same 3xTF32 tcgen05 pipeline as the forward), store the pre-BN
+//   head   : recompute the conditioner (3xTF32 tcgen05 pipeline, that of the round-1 forward), store the pre-BN
 //            activations z_1..z_depth, run the spline forward + hand-derived spline backward on the logits
 //            in registers -> dL/dlogits (stored), dL/dx of the transformed columns, dL/dJ
 //   layer  : one launch per linear layer lam = depth (output layer) .. 0.  Upstream gradient dz (logits
@@ -23,7 +23,7 @@
 // along M ([dz_hi ; dz_lo], 128 rows) so that two M=128 MMAs (against h_hi and h_lo) give all four partial
 // products; rows o and 64+o of the accumulator are added on read-out.
 //
-// Same CTA shape as the forward (8 point warps + one MMA-issuing warp); in the layer launches the 8 warps work
+// CTA of 8 point warps (two 128-point groups) + one MMA-issuing warp; in the layer launches the 8 warps work
 // on ONE tile, two threads per point (see flow_bwd_tc_layer_kernel).
 #include <stdlib.h>
 #include "common.cuh"
@@ -41,7 +41,7 @@ struct BtArgs {
     void* grad_in;
     float* gstate;                         // [B][d+1]
     const float* params; const float* wpack; const float* bn_saved;
-    const float* tcpack;                   // forward operands (flow_tc.cu pack)
+    const float* tcpack;                   // forward operands (flow_tc_pack_kernel)
     const float* bdpack;                   // dgrad operands (W^T hi/lo)
     float* zbuf;                           // [depth][tiles][64][128] pre-BN activations z_1..z_depth
     float* dl;                             // [tiles][128][128] dL/dlogits
@@ -54,6 +54,44 @@ struct BtArgs {
     int c, lam, first, grid;
     int flush_every;                       // iterations between flushes of the wgrad accumulators (0: only at the end)
 };
+
+// Operands of the head's conditioner recompute: hidden layers 1..depth-1 and the output blocks, each as TF32 hi / lo
+// splits in the K-major 128-byte-swizzled layout, tc_cell_floats(F) per cell (tc_common.cuh)
+__global__ void flow_tc_pack_kernel(DevFlow F, const float* __restrict__ params, float* __restrict__ tcpack) {
+    const int c = blockIdx.y;
+    const DevCell& q = F.cells[c];
+    const float* p = params + q.param_off;
+    char* dst = reinterpret_cast<char*>(tcpack + (size_t)c * tc_cell_floats(F));
+    const int tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
+    for (int l = 1; l < F.depth; ++l) {
+        const float* w = p + F.p_lin(c, l);                     // [64][64] torch layout (out, in)
+        char* hi = dst + (size_t)(l - 1) * 2 * TCH * TCH * 4;
+        char* lo = hi + (size_t)TCH * TCH * 4;
+        for (int i = tid; i < TCH * TCH; i += nth) {
+            const int n = i / TCH, k = i - n * TCH;
+            const float v = w[(size_t)n * TCH + k];
+            const float h = tf32_rn(v);
+            const int o = tc_off(TCH, n, k);
+            *reinterpret_cast<float*>(hi + o) = h;
+            *reinterpret_cast<float*>(lo + o) = tf32_rn(v - h);
+        }
+    }
+    const float* wo = p + F.p_lin(c, F.depth);                  // [T*K][64]
+    const int Nb = tc_out_n(F), tper = tc_out_tper(F), slot = tc_out_slot(F);
+    for (int b = 0; b < tc_out_blocks(F, q.T); ++b) {
+        char* hi = dst + (size_t)(F.depth - 1) * 2 * TCH * TCH * 4 + (size_t)b * 2 * Nb * TCH * 4;
+        char* lo = hi + (size_t)Nb * TCH * 4;
+        for (int i = tid; i < Nb * TCH; i += nth) {
+            const int n = i / TCH, k = i - n * TCH;
+            const int t = b * tper + n / slot, jj = n % slot;
+            const float v = (t < q.T && jj < F.K) ? wo[((size_t)t * F.K + jj) * TCH + k] : 0.f;
+            const float h = tf32_rn(v);
+            const int o = tc_off(Nb, n, k);
+            *reinterpret_cast<float*>(hi + o) = h;
+            *reinterpret_cast<float*>(lo + o) = tf32_rn(v - h);
+        }
+    }
+}
 
 __host__ __device__ static inline int bd_layer_off(const DevFlow& F, int lam) {      // floats, inside a cell's block
     return lam == 0 ? 0 : 2 * 16 * TCH + (lam - 1) * 2 * TCH * TCH;
@@ -827,8 +865,41 @@ __global__ void flow_bwd_tc_reduce_kernel(DevFlow F, const float* __restrict__ s
 }
 
 // ---------------------------------------------------------------------------------------------------
-bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_tc_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s);
+size_t nis_tc_pack_floats(const DevFlow& F) {
+    if (F.depth < 1) return 0;
+    return (size_t)F.n_cells * tc_cell_floats(F);
+}
+
+int nis_tc_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s) {
+    flow_tc_pack_kernel<<<dim3(16, F.n_cells), 256, 0, s>>>(F, params, tcpack);
+    NIS_CUDA_CHECK_LAUNCH();
+    return NIS_OK;
+}
+
+int64_t nis_tc_min_batch(int64_t dflt);
+
+// Width-64 cells with 32 bins (PWLin or PWQuad) whose operands in the 3xTF32 layout (tc_layout) fit an SM's shared memory
+// in each launch shape of the round-1 forward: fused eval cell, layer pass, final pass.  The tensor-core backward below
+// takes the PWLin ones; flow_fwd.cu runs the fp16-split forward and inverse only on shapes this accepts.
+bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode) {
+    (void)bn_mode;
+    const char* off = getenv("NIS_TC");                   // NIS_TC=0 forces the FP32-pipe kernels (test knob)
+    if (off && off[0] == '0') return false;
+    if (F.depth < 1 || B < nis_tc_min_batch(256) || F.maxW != TCH || F.nb != 32) return false;
+    for (int l = 0; l < F.depth; ++l) if (F.widths[l] != TCH) return false;
+    if (F.kind == NIS_KIND_PWLIN ? F.K != 32 : F.K != 65) return false;
+    for (int c = 0; c < F.n_cells; ++c) {
+        const int P = F.cells[c].P, T = F.cells[c].T;
+        if (P > 16) return false;
+        if (F.K == 32 && T * 32 > TC_NOUT) return false;
+        const size_t lim = 226 * 1024;
+        if ((size_t)tc_layout(F, P, 1, F.depth, false).total + 1024 > lim && F.K == 32) return false;      // fused eval cell
+        if ((size_t)tc_layout(F, P, 1, F.depth - 1, true).total + 1024 > lim) return false;               // hidden pass(es)
+        if ((size_t)tc_layout(F, P, F.depth, F.depth, F.K == 32).total + 1024 > lim) return false;        // final pass
+    }
+    return true;
+}
+
 __global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_running,
                                  float* __restrict__ wpack, int bn_mode);
 

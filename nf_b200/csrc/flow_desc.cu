@@ -100,7 +100,8 @@ size_t nis_flow_carve(const DevFlow& F, int64_t B, void* base, FlowWorkspace* ws
     size_t off = 0;
     char* b = (char*)base;
     ws->wpack = (float*)(b + off); off = align256(off + sizeof(float) * (size_t)F.pack_total);
-    {   // tensor-core operand pack: resident-weights layout (flow_tc.cu) or K-panels (flow_wide.cu)
+    {   // tensor-core operand pack: 3xTF32 resident-weights layout (flow_bwd_tc.cu), which also holds the fp16-split one
+        // (flow_tc_h.cu), or K-panels (flow_wide.cu)
         size_t fl = nis_tc_pack_floats(F), wf = nis_wide_pack_floats(F);
         ws->tcpack = (float*)(b + off); off = align256(off + sizeof(float) * (fl > wf ? fl : wf));
     }

@@ -285,9 +285,6 @@ size_t nis_flow_bwd_scratch_floats(const DevFlow& F, int64_t B);
 bool nis_tiled_supported(const DevFlow& F, int64_t B);
 size_t nis_tiled_zbuf_floats(int64_t B);
 bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_tc_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s);
-int nis_launch_tc(const DevFlow& F, const FwdArgs& A, const float* tcpack, cudaStream_t s);
-bool nis_tc_split_eval(const DevFlow& F);
 bool nis_h_supported(const DevFlow& F, int64_t B, int bn_mode);
 int nis_h_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s);
 int nis_launch_h(const DevFlow& F, const FwdArgs& A, const float* tcpack, cudaStream_t s);
@@ -438,6 +435,69 @@ extern "C" int64_t nis_flow_act_saved_count(const NisFlowDesc* desc, int64_t B) 
     return (int64_t)nis_act_cache_floats(F, B);
 }
 
+// The fp16-split kernel (flow_tc_h.cu) runs the width-64 PWLin / PWQuad flows with 32 bins that nis_tc_supported accepts,
+// the gate of the tensor-core backward; nis_h_supported accepts all of them.  On its own it would accept about five times
+// as many shapes (for example every n_flow >= 10 at depth 1), which run on the streamed-weights kernel (flow_wide.cu) today:
+// giving them to the fp16-split kernel needs parity tests and B200 timings against that kernel of their own.
+static bool h_path(const DevFlow& F, int64_t B, int bn_mode) { return nis_tc_supported(F, B, bn_mode) && nis_h_supported(F, B, bn_mode); }
+
+// One cell on the fp16-split kernel, forward or inverse (A.inverse).  Train mode: BN_0 and BN_1 from the column moments
+// unless the previous cell's final pass has taken them (moments_ready), then a layer pass per remaining BN layer.  With
+// depth >= 3 PWLin cells the last layer pass only takes the statistics of z_depth (no 256 B/point store) and the final pass
+// starts from z_{depth-1} and runs the last hidden layer again: 7.74 -> 7.29 ms on cfg2 (the PWQuad final pass is bound by
+// its spline and loses 1 %).  The final pass reads the state rows from state_in (nullptr: the input rows A.in) and writes
+// them to state_out and, with to_out, to A.out; it also takes the column moments of cell `next` (-1: none) when that cell
+// has P <= 4, and moments_ready tells the next call whether it did.
+static int h_cell(const DevFlow& F, FwdArgs& A, const FlowWorkspace& ws, int bn_mode, int c, int next, const float* state_in,
+                  float* state_out, bool to_out, bool& moments_ready, cudaStream_t s) {
+    const bool train = bn_mode == NIS_BN_TRAIN;
+    const bool moments = train && nis_moments_supported(F, c);
+    const bool skip_last = moments && F.depth >= 3 && F.kind == NIS_KIND_PWLIN;
+    float* zb[2] = {ws.bwd, ws.bwd + zbuf_floats(F, A.B)};
+    A.c_begin = c; A.c_end = c + 1;
+    A.from_state = state_in != nullptr; A.state_in = state_in;
+    A.state_out = nullptr; A.to_out = 0;
+    A.zin_layer = 0; A.next_moments = 0;
+    int rc;
+    if (train) {
+        int l0 = 0;
+        if (moments) {
+            if (!moments_ready) {
+                A.stats_layer = 0;
+                rc = nis_launch_col_moments(F, A, s);
+                if (rc) return rc;
+                timing_mark(s, 1);
+            }
+            l0 = 2;
+        }
+        for (int l = l0; l <= F.depth; ++l) {
+            A.stats_layer = l;
+            if (l >= 1) {
+                // layer pass: reads the pre-BN activations of layer l-1, writes those of layer l
+                A.zin = (l >= 2 && !(moments && l == 2)) ? zb[(l - 1) & 1] : nullptr;
+                A.zout = (skip_last && l == F.depth) ? nullptr : zb[l & 1];
+                rc = nis_launch_h(F, A, ws.tcpack, s);
+            } else {
+                rc = nis_launch_col_stats(F, A, s);
+            }
+            if (rc) return rc;
+            timing_mark(s, l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
+        }
+    }
+    A.stats_layer = -1;
+    A.zin = (train && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
+    A.zout = nullptr;
+    if (skip_last) { A.zin = zb[(F.depth - 1) & 1]; A.zin_layer = F.depth - 1; }
+    A.next_moments = train && next >= 0 && A.zin != nullptr && nis_moments_supported(F, next) && F.cells[next].P <= 4;
+    A.next_cell = next;
+    moments_ready = A.next_moments != 0;
+    A.state_out = state_out; A.to_out = to_out;
+    rc = nis_launch_h(F, A, ws.tcpack, s);
+    if (rc) return rc;
+    timing_mark(s, 10 + (A.zin ? 2 : 0));
+    return NIS_OK;
+}
+
 extern "C" int nis_flow_forward(const NisFlowDesc* desc, const float* params, float* bn_running,
                                 const void* xj_in, int32_t in_dtype, int32_t in_cols,
                                 void* xj_out, int32_t out_dtype, int32_t* bins_out,
@@ -485,24 +545,25 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
     A.params = params; A.wpack = ws.wpack; A.bn_running = bn_running; A.bn_saved = bn_saved;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B;
     A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 0; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
-    // per-cell launch sequences: tcgen05 kernel where it applies, else the FP32 register-tiled kernel
-    const bool tc = nis_tc_supported(F, B, bn_mode);
-    const bool hp = tc && nis_h_supported(F, B, bn_mode);              // fp16-split, four-group kernel (flow_tc_h.cu)
-    const bool wide = !tc && nis_wide_supported(F, B, bn_mode);       // streamed-weights tcgen05 kernel (flow_wide.cu)
-    const bool tiled = tc || wide || nis_tiled_supported(F, B);
-    // train-mode layer passes either hand their pre-BN activations to the next pass through HBM (256 B/point/pass) or
-    // recompute them from the state (more tensor work, ~7x less traffic); NIS_TRAIN_RECOMPUTE=0/1 overrides the default
-    static const int recompute_env = [] { const char* e = getenv("NIS_TRAIN_RECOMPUTE"); return e ? (e[0] == '1' ? 1 : 0) : -1; }();
-    const bool recompute = hp && (recompute_env >= 0 ? recompute_env == 1 : false);
-    // fp16-split kernel, depth >= 3: the last layer pass only takes the statistics of z_depth (no 256 B/point store) and the final
-    // pass starts from z_{depth-1} and runs the last hidden layer again (one more MMA block per tile, 256 B/point less traffic
-    // per cell); NIS_SKIP_LAST_STORE=0 keeps the store (A/B knob)
-    static const int skip_env = [] { const char* e = getenv("NIS_SKIP_LAST_STORE"); return e && e[0] == '0' ? 0 : 1; }();
-    // (PWLin only: measured 7.74 -> 7.29 ms on cfg2; the PWQuad final pass is instruction-bound on its spline and loses 1 %)
-    const bool skip_last = hp && !recompute && skip_env && F.depth >= 3 && F.kind == NIS_KIND_PWLIN;
-    if (tc) { rc = hp ? nis_h_pack(F, params, ws.tcpack, s) : nis_tc_pack(F, params, ws.tcpack, s); if (rc) return rc; timing_mark(s, 0); }
-    if (wide) { rc = nis_wide_pack(F, params, ws.tcpack, s); if (rc) return rc; }
     const long long rows = (long long)B * (F.d + 1);
+    if (h_path(F, B, bn_mode)) {
+        rc = nis_h_pack(F, params, ws.tcpack, s);
+        if (rc) return rc;
+        timing_mark(s, 0);
+        bool moments_ready = false;
+        for (int c = 0; c < F.n_cells; ++c) {
+            const bool last = c == F.n_cells - 1;
+            rc = h_cell(F, A, ws, bn_mode, c, last ? -1 : c + 1, c > 0 ? (saved ? saved + c * rows : ws.state) : nullptr,
+                        saved ? saved + (c + 1) * rows : (last ? nullptr : ws.state), last, moments_ready, s);
+            if (rc) return rc;
+        }
+        return NIS_OK;
+    }
+    // every other shape: streamed-weights tcgen05 kernel (flow_wide.cu), else the FP32 register-tiled kernel, else the
+    // shape-generic one
+    const bool wide = nis_wide_supported(F, B, bn_mode);
+    const bool tiled = wide || nis_tiled_supported(F, B);
+    if (wide) { rc = nis_wide_pack(F, params, ws.tcpack, s); if (rc) return rc; }
     if (bn_mode == NIS_BN_EVAL && !tiled) {
         A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 1;
         A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
@@ -519,16 +580,12 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
             if (rc == NIS_OK) { timing_mark(s, 2); return NIS_OK; }
         }
     }
-    // fp16-split kernel: the final pass of a train-mode cell also takes the column moments of the next cell (P <= 4) from the
-    // state it writes, so only the first cell runs flow_col_moments_kernel (NIS_FUSE_MOMENTS=0: every cell does, A/B knob)
-    static const int fuse_env = [] { const char* e = getenv("NIS_FUSE_MOMENTS"); return e && e[0] == '0' ? 0 : 1; }();
-    bool moments_ready = false;
     // activation cache (nis_flow_forward_cached): the wide layer passes write z_1..z_depth of every cell there instead of the
     // two rotating workspace buffers
     float* acts = (wide && bn_mode == NIS_BN_TRAIN && act_saved && saved && nis_act_cache_floats(F, B)) ? act_saved : nullptr;
     const size_t act_layer = (size_t)((B + 127) / 128) * (size_t)F.widths[0] * 128;
     // One launch sequence per cell.  TRAIN: a statistics pass per BN layer, then the full pass.
-    // (EVAL reaches here only on the register-tiled path, whose launches are per cell.)
+    // (EVAL reaches here only on the register-tiled and streamed-weights paths, whose launches are per cell.)
     for (int c = 0; c < F.n_cells; ++c) {
         A.c_begin = c; A.c_end = c + 1;
         A.from_state = c > 0;
@@ -542,48 +599,37 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
         if (bn_mode == NIS_BN_TRAIN) {
             int l0 = 0;
             if (moments) {
-                if (!moments_ready) {
-                    A.stats_layer = 0;
-                    rc = nis_launch_col_moments(F, A, s);
-                    if (rc) return rc;
-                    timing_mark(s, 1);
-                }
+                A.stats_layer = 0;
+                rc = nis_launch_col_moments(F, A, s);
+                if (rc) return rc;
+                timing_mark(s, 1);
                 l0 = 2;
             }
             for (int l = l0; l <= F.depth; ++l) {
                 A.stats_layer = l;
                 if (tiled && l >= 1) {
                     // layer pass: reads the pre-BN activations of layer l-1, writes those of layer l
-                    A.zin = (l >= 2 && !(moments && l == 2) && !recompute) ? zb[(l - 1) & 1] : nullptr;
-                    A.zout = (recompute || (skip_last && moments && l == F.depth)) ? nullptr : zb[l & 1];
+                    A.zin = (l >= 2 && !(moments && l == 2)) ? zb[(l - 1) & 1] : nullptr;
+                    A.zout = zb[l & 1];
                     if (acell) {
                         if (A.zin) A.zin = acell + (size_t)(l - 2) * act_layer;
                         A.zout = acell + (size_t)(l - 1) * act_layer;
                         A.z1out = (!A.zin && l == 2) ? acell : nullptr;
                     }
-                    rc = hp ? nis_launch_h(F, A, ws.tcpack, s) : tc ? nis_launch_tc(F, A, ws.tcpack, s)
-                            : wide ? nis_launch_wide(F, A, ws.tcpack, s) : nis_launch_tiled(F, A, s);
+                    rc = wide ? nis_launch_wide(F, A, ws.tcpack, s) : nis_launch_tiled(F, A, s);
                 } else if (tiled && l == 0) {
                     rc = nis_launch_col_stats(F, A, s);
                 } else {
                     rc = launch_fwd_any(F, A, s);
                 }
                 if (rc) return rc;
-                timing_mark(s, (tc || wide) && l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
+                timing_mark(s, wide && l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
             }
         }
         A.stats_layer = -1;
-        A.zin = (tiled && bn_mode == NIS_BN_TRAIN && !(moments && F.depth == 1) && !recompute) ? zb[F.depth & 1] : nullptr;
+        A.zin = (tiled && bn_mode == NIS_BN_TRAIN && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
         A.zout = nullptr;
         if (acell) { A.zin = acell + (size_t)(F.depth - 1) * act_layer; A.z1out = nullptr; }
-        if (skip_last && moments && bn_mode == NIS_BN_TRAIN) { A.zin = zb[(F.depth - 1) & 1]; A.zin_layer = F.depth - 1; }
-        if (tc && !hp && bn_mode == NIS_BN_EVAL && nis_tc_split_eval(F)) {
-            // eval, PWQuad: hidden layers in one launch (activations of the last hidden layer to HBM), then the final pass
-            A.stats_layer = F.depth; A.no_stats = 1; A.zin = nullptr; A.zout = zb[F.depth & 1];
-            rc = nis_launch_tc(F, A, ws.tcpack, s);
-            if (rc) return rc;
-            A.stats_layer = -1; A.no_stats = 0; A.zin = zb[F.depth & 1]; A.zout = nullptr;
-        }
         if (wide && bn_mode == NIS_BN_EVAL) {
             // eval, wide conditioner: one launch per hidden layer (no statistics), then the final pass
             A.no_stats = 1;
@@ -597,17 +643,11 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
             A.stats_layer = -1; A.no_stats = 0; A.zin = F.depth >= 2 ? zb[F.depth & 1] : nullptr; A.zout = nullptr;
         }
         const bool last = c == F.n_cells - 1;
-        A.next_moments = hp && fuse_env && bn_mode == NIS_BN_TRAIN && !last && A.zin != nullptr
-                         && nis_moments_supported(F, c + 1) && F.cells[c + 1].P <= 4;
-        A.next_cell = c + 1;
-        moments_ready = A.next_moments != 0;
         A.to_out = last;
         A.state_out = saved ? saved + (long long)(c + 1) * rows : (last ? nullptr : ws.state);
-        rc = hp ? nis_launch_h(F, A, ws.tcpack, s) : tc ? nis_launch_tc(F, A, ws.tcpack, s) : wide ? nis_launch_wide(F, A, ws.tcpack, s)
-                : (tiled ? nis_launch_tiled(F, A, s) : launch_fwd_any(F, A, s));
+        rc = wide ? nis_launch_wide(F, A, ws.tcpack, s) : tiled ? nis_launch_tiled(F, A, s) : launch_fwd_any(F, A, s);
         if (rc) return rc;
-        timing_mark(s, (tc || wide) ? 10 + (A.zin ? 2 : 0) : 2);
-        A.zin_layer = 0;
+        timing_mark(s, wide ? 10 + (A.zin ? 2 : 0) : 2);
     }
     return NIS_OK;
 }
@@ -632,73 +672,6 @@ __global__ void __launch_bounds__(256) flow_inverse_gather_kernel(const __grid_c
         const float v = (r < d || in_cols > d) ? load_io(in, in_dtype, pt * in_cols + r) : 1.f;
         state[pt * (d + 1) + (r < d ? F.out_perm[r] : d)] = v;
     }
-}
-
-// The inverse on the fp16-split kernel: the forward's launch sequence with the cells in reverse order.  The statistics and
-// layer passes are the forward's (they read only the pass-through columns); the fused cell and the final pass run the
-// inverse splines; the fused column moments of a final pass are those of cell c - 1.
-static int inverse_h(const DevFlow& F, FwdArgs A, const FlowWorkspace& ws, int bn_mode, cudaStream_t s) {
-    const long long B = A.B;
-    int rc = nis_h_pack(F, A.params, ws.tcpack, s);
-    if (rc) return rc;
-    timing_mark(s, 0);
-    {
-        const long long n = B * (F.d + 1);
-        const long long nb = (n + 255) / 256;
-        flow_inverse_gather_kernel<<<(unsigned)(nb < 4096 ? nb : 4096), 256, 0, s>>>(F, A.in, A.in_dtype, A.in_cols, B, ws.state);
-        NIS_CUDA_CHECK_LAUNCH();
-        timing_mark(s, 2);
-    }
-    const bool train = bn_mode == NIS_BN_TRAIN;
-    static const int skip_env = [] { const char* e = getenv("NIS_SKIP_LAST_STORE"); return e && e[0] == '0' ? 0 : 1; }();
-    static const int fuse_env = [] { const char* e = getenv("NIS_FUSE_MOMENTS"); return e && e[0] == '0' ? 0 : 1; }();
-    const bool skip_last = skip_env && F.depth >= 3 && F.kind == NIS_KIND_PWLIN;
-    float* zb[2] = {ws.bwd, ws.bwd + zbuf_floats(F, B)};
-    A.from_state = 1; A.state_in = ws.state;
-    bool moments_ready = false;
-    for (int c = F.n_cells - 1; c >= 0; --c) {
-        A.c_begin = c; A.c_end = c + 1;
-        A.state_out = nullptr; A.to_out = 0;
-        A.zin = nullptr; A.zout = nullptr; A.zin_layer = 0; A.next_moments = 0;
-        const bool moments = train && nis_moments_supported(F, c);
-        if (train) {
-            int l0 = 0;
-            if (moments) {
-                if (!moments_ready) {
-                    A.stats_layer = 0;
-                    rc = nis_launch_col_moments(F, A, s);
-                    if (rc) return rc;
-                    timing_mark(s, 1);
-                }
-                l0 = 2;
-            }
-            for (int l = l0; l <= F.depth; ++l) {
-                A.stats_layer = l;
-                if (l >= 1) {
-                    A.zin = (l >= 2 && !(moments && l == 2)) ? zb[(l - 1) & 1] : nullptr;
-                    A.zout = (skip_last && moments && l == F.depth) ? nullptr : zb[l & 1];
-                    rc = nis_launch_h(F, A, ws.tcpack, s);
-                } else {
-                    rc = nis_launch_col_stats(F, A, s);
-                }
-                if (rc) return rc;
-                timing_mark(s, l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
-            }
-        }
-        A.stats_layer = -1;
-        A.zin = (train && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
-        A.zout = nullptr;
-        if (skip_last && moments) { A.zin = zb[(F.depth - 1) & 1]; A.zin_layer = F.depth - 1; }
-        A.next_moments = fuse_env && train && c > 0 && A.zin != nullptr && nis_moments_supported(F, c - 1) && F.cells[c - 1].P <= 4;
-        A.next_cell = c - 1;
-        moments_ready = A.next_moments != 0;
-        A.to_out = c == 0;
-        A.state_out = c == 0 ? nullptr : ws.state;
-        rc = nis_launch_h(F, A, ws.tcpack, s);
-        if (rc) return rc;
-        timing_mark(s, 10 + (A.zin ? 2 : 0));
-    }
-    return NIS_OK;
 }
 
 extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, const float* bn_running,
@@ -738,7 +711,24 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
     A.params = params; A.wpack = ws.wpack; A.bn_running = nullptr; A.bn_saved = nullptr;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B;
     A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 1; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
-    if (nis_tc_supported(F, B, bn_mode) && nis_h_supported(F, B, bn_mode)) return inverse_h(F, A, ws, bn_mode, s);
+    if (h_path(F, B, bn_mode)) {
+        // the forward's launch sequence with the cells in reverse order, from float32 state rows in the physical column
+        // order.  The statistics and layer passes are the forward's (they read only the pass-through columns); the fused
+        // cell and the final pass run the inverse splines; the fused column moments of a final pass are those of cell c - 1.
+        rc = nis_h_pack(F, params, ws.tcpack, s);
+        if (rc) return rc;
+        timing_mark(s, 0);
+        const long long nb = (B * (F.d + 1) + 255) / 256;
+        flow_inverse_gather_kernel<<<(unsigned)(nb < 4096 ? nb : 4096), 256, 0, s>>>(F, yj_in, in_dtype, in_cols, B, ws.state);
+        NIS_CUDA_CHECK_LAUNCH();
+        timing_mark(s, 2);
+        bool moments_ready = false;
+        for (int c = F.n_cells - 1; c >= 0; --c) {
+            rc = h_cell(F, A, ws, bn_mode, c, c - 1, ws.state, c == 0 ? nullptr : ws.state, c == 0, moments_ready, s);
+            if (rc) return rc;
+        }
+        return NIS_OK;
+    }
     if (bn_mode == NIS_BN_EVAL) {
         A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 1;
         A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;

@@ -1,5 +1,5 @@
-// Fused coupling-cell forward, width-64 PWLin cells, on tcgen05 with a HALF-PRECISION SPLIT of the operands —
-// the round-2 successor of flow_tc.cu's 3xTF32 kernel (which stays for PWQuad cells and as the A/B reference).
+// Fused coupling-cell forward and inverse, width-64 PWLin and PWQuad cells with 32 bins, on tcgen05 with a HALF-PRECISION
+// SPLIT of the operands — the round-2 successor of the round-1 3xTF32 kernel (since removed, DESIGN.md 4.3a).
 //
 // Why: ncu on the 3xTF32 kernel (profiles/r01_ncu_tc.md) showed a latency-bound chain epilogue -> MMA -> epilogue
 // with only TWO 128-point groups per SM to overlap (warp slots 14 % occupied, 52 % of the stall samples on the
@@ -17,8 +17,8 @@
 //   * there is no issuer warp: thread 0 of a group issues the group's own MMAs once the group's 128 "my operand row
 //     is in tensor memory" arrivals are in (a 17th warp would cap the kernel at 96 registers per thread, and a
 //     group never queues behind a slower one).
-// The layer-pass scheme for train-mode BatchNorm, the tile-blocked activation buffers and the statistics fold are
-// those of flow_tc.cu / flow_tiled.cu (DESIGN.md 4.2b).  Reference: coupling_cells.py:84-142 (PWLin + conditioner).
+// The layer-pass scheme for train-mode BatchNorm and the tile-blocked activation buffers are those of flow_tiled.cu
+// (DESIGN.md 4.2b).  Reference: coupling_cells.py:84-142 (PWLin + conditioner), :159-228 (PWQuad).
 #include <stdlib.h>
 #include <cuda_fp16.h>
 #include "common.cuh"
@@ -218,7 +218,7 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
     const int c = A.c_begin;
     const DevCell& q = F.cells[c];
     const int d = F.d, depth = F.depth;
-    // which slice of the cell this launch computes (same table as flow_tc.cu)
+    // which slice of the cell this launch computes (MODE, above)
     constexpr bool stats = (MODE & 1) != 0;
     constexpr bool from_z = (MODE & 2) != 0;
     constexpr bool nextmom = (MODE & 4) != 0;
@@ -561,8 +561,8 @@ __global__ void __launch_bounds__(NG * TCM, 1) flow_cell_h_kernel(const __grid_c
                     for (int j = 0; j < 65; ++j) z[j] = fmaf(z[j], inv_out, bs[j]);
                     float y, f;
                     int kb;
-                    if (inverse) pwquad32_tree_inv<true>(z, xv, y, f, kb);      // (f = 1 / density)
-                    else pwquad32_tree<true>(z, xv, y, f, kb);
+                    if (inverse) pwquad32_tree_inv(z, xv, y, f, kb);      // (f = 1 / density)
+                    else pwquad32_tree(z, xv, y, f, kb);
                     st[q.trafo[b] * TCM] = y;
                     jfac *= f;
                     if (A.bins && valid) A.bins[((long long)c * A.B + pt) * d + b] = kb;
@@ -652,7 +652,11 @@ size_t nis_h_pack_floats(const DevFlow& F) {
     return (size_t)F.n_cells * (h_cell_bytes(F) / 4);
 }
 
-int64_t nis_tc_min_batch(int64_t dflt);
+// smallest batch the tensor-core kernels take (below it the shape-generic kernel runs); NIS_TC_MIN_B overrides (test knob)
+int64_t nis_tc_min_batch(int64_t dflt) {
+    const char* e = getenv("NIS_TC_MIN_B");
+    return e ? atoll(e) : dflt;
+}
 
 static int h_groups(const DevFlow& F) {
     // the largest group count whose three launch shapes fit the shared memory of an SM
@@ -671,12 +675,9 @@ static int h_groups(const DevFlow& F) {
     return 0;
 }
 
-// Width-64 cells with 32 bins: PWLin (BASELINE configs[1]) and PWQuad (configs[3]); NIS_TC_H=0 keeps the 3xTF32 kernel
-// (A/B test knob)
+// Width-64 cells with 32 bins: PWLin (BASELINE configs[1]) and PWQuad (configs[3])
 bool nis_h_supported(const DevFlow& F, int64_t B, int bn_mode) {
     (void)bn_mode;
-    const char* off = getenv("NIS_TC_H");
-    if (off && off[0] == '0') return false;
     const char* tcoff = getenv("NIS_TC");
     if (tcoff && tcoff[0] == '0') return false;
     if (F.nb != 32 || F.depth < 1 || F.maxW != TCH) return false;

@@ -58,8 +58,11 @@ __host__ __device__ static inline TiledSmem tiled_layout(const DevFlow& F, int c
 template <int M>
 __device__ __forceinline__ int swz(int row, int pt) { return row * M + ((((pt >> 2) ^ ((row >> 2) & 7)) << 2) | (pt & 3)); }
 
-template <int M, int TM>
-__global__ void __launch_bounds__(M * 8 / TM, (M == 128 && TM == 4) ? 2 : 1) flow_cell_tiled_kernel(const __grid_constant__ DevFlow F, const FwdArgs A) {
+// 4x8 register tiles (16 warps/SM) measured faster than 8x8 (8 warps/SM) on B200: 26.0 vs 29.0 ms for cfg2 eval at 2^22 points
+constexpr int TM = 4;
+
+template <int M>
+__global__ void __launch_bounds__(M * 8 / TM, M == 128 ? 2 : 1) flow_cell_tiled_kernel(const __grid_constant__ DevFlow F, const FwdArgs A) {
     constexpr int NT = M * 8 / TM;
     constexpr int NV = TM / 4;            // float4 per thread row
     extern __shared__ __align__(16) float sm[];
@@ -481,18 +484,18 @@ bool nis_tiled_supported(const DevFlow& F, int64_t B) {
     return true;
 }
 
-template <int M, int TM>
+template <int M>
 static int launch_tiled_m(const DevFlow& F, const FwdArgs& A, int sms, cudaStream_t s) {
     const bool stats = A.stats_layer >= 1;
     const int last = stats ? A.stats_layer : F.depth;
     const int first = A.zin ? last - (stats ? 1 : 0) : 0;
     TiledSmem L = tiled_layout(F, A.c_begin, M, first, last, !stats);
     const size_t smem = (size_t)L.total * sizeof(float);
-    NIS_ENSURE_SMEM((flow_cell_tiled_kernel<M, TM>), (int)smem);
+    NIS_ENSURE_SMEM((flow_cell_tiled_kernel<M>), (int)smem);
     long long ntiles = (A.B + M - 1) / M;
-    const int per_sm = (M == 128 && TM == 4 && smem <= 110 * 1024) ? 2 : 1;
+    const int per_sm = (M == 128 && smem <= 110 * 1024) ? 2 : 1;
     int grid = (int)(ntiles < (long long)sms * per_sm ? ntiles : (long long)sms * per_sm);
-    flow_cell_tiled_kernel<M, TM><<<grid, M * 8 / TM, smem, s>>>(F, A);
+    flow_cell_tiled_kernel<M><<<grid, M * 8 / TM, smem, s>>>(F, A);
     NIS_CUDA_CHECK_LAUNCH();
     return NIS_OK;
 }
@@ -506,11 +509,6 @@ int nis_launch_tiled(const DevFlow& F, const FwdArgs& A, cudaStream_t s) {
     // same M; they run at M=128 with two CTAs per SM.  The fused eval cell runs at M=256.
     const bool layer_pass = A.zin || A.zout;
     TiledSmem L256 = tiled_layout(F, A.c_begin, 256, 0, F.depth, true);
-    // 4x8 register tiles (16 warps/SM) measured faster than 8x8 (8 warps/SM) on B200: 26.0 vs 29.0 ms for
-    // cfg2 eval at 2^22 points; NIS_TILED_VARIANT=8 selects the 8x8 variant for experiments.
-    const char* v = getenv("NIS_TILED_VARIANT");
-    const bool tm4 = !(v && v[0] == '8');
-    if (!layer_pass && (size_t)L256.total * 4 <= 225 * 1024 && A.B >= (long long)sms * 256)
-        return tm4 ? launch_tiled_m<256, 4>(F, A, sms, s) : launch_tiled_m<256, 8>(F, A, sms, s);
-    return tm4 ? launch_tiled_m<128, 4>(F, A, sms, s) : launch_tiled_m<128, 8>(F, A, sms, s);
+    if (!layer_pass && (size_t)L256.total * 4 <= 225 * 1024 && A.B >= (long long)sms * 256) return launch_tiled_m<256>(F, A, sms, s);
+    return launch_tiled_m<128>(F, A, sms, s);
 }

@@ -2,7 +2,7 @@
 // BASELINE configs[4]: 16-D PWQuad, 64 bins, MLP [256]*4, where the conditioner is a real dense contraction
 // (7.4 MFLOP per point).
 //
-// A 256-wide layer does not fit the resident-weights scheme of flow_tc.cu (one layer's hi/lo operand is
+// A 256-wide layer does not fit the resident-weights scheme of flow_tc_h.cu (one layer's hi/lo operand is
 // 512 KB), so the layer runs as a streamed GEMM per 128-point tile:
 //   * weights are packed once per forward as K-panels of 32 input features, [N rows][32] hi then lo in the
 //     K-major 128B-swizzled UMMA layout, and STREAMED from L2 through a ring of shared-memory slots by
@@ -17,7 +17,7 @@
 //     the float64 oracle as torch-fp32).  The hi*hi products (32 steps) go to D_hi, the two cross products
 //     (2^-11 smaller, so their truncation does not matter) to D_x, and the epilogue adds the two in fp32.
 //     N <= 192 per round (2 x 192 accumulator columns); a 256-wide layer is two rounds of 128 outputs.
-// One launch = one layer of one cell (the train-mode layer-pass scheme of flow_tiled.cu / flow_tc.cu, which
+// One launch = one layer of one cell (the train-mode layer-pass scheme of flow_tiled.cu / flow_tc_h.cu, which
 // also serves eval mode here: activations round-trip through HBM tile-blocked [tile][W][128], 1 KB/point/layer,
 // far below the tensor time).  The final pass runs the output layer one transformed dimension at a time
 // (N = K logits padded to 16), stages the logits in shared memory and runs the spline of spline.cuh on them.
@@ -386,7 +386,7 @@ bool nis_wide_supported(const DevFlow& F, int64_t B, int bn_mode) {
     if (off && off[0] == '0') return false;
     if (F.depth < 1 || B < nis_tc_min_batch(256) || F.kind == NIS_KIND_AFFINE) return false;
     const int W = F.widths[0];
-    if (W < 64 || W > 256 || (W & 63)) return false;          // (width 64 with 32 bins is taken by flow_tc.cu first)
+    if (W < 64 || W > 256 || (W & 63)) return false;          // (width 64 with 32 bins is taken by flow_tc_h.cu first where it applies)
     for (int l = 0; l < F.depth; ++l) if (F.widths[l] != W) return false;
     if (F.maxW != W) return false;
     if (wd_kp16(F) > WD_NMAX) return false;

@@ -1,6 +1,6 @@
-// tcgen05 / TMEM / bulk-copy building blocks shared by the tensor-core flow kernels (flow_tc.cu forward,
-// flow_bwd_tc.cu backward): PTX wrappers, the K-major 128-byte-swizzled operand layout, TMEM <-> register
-// moves, the 3xTF32 split.
+// tcgen05 / TMEM / bulk-copy building blocks shared by the tensor-core flow kernels (flow_tc_h.cu, flow_wide.cu
+// forward; flow_bwd_tc.cu, flow_bwd_wide.cu backward): PTX wrappers, the K-major 128-byte-swizzled operand layout,
+// TMEM <-> register moves, the 3xTF32 split.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

@@ -1,60 +1,7 @@
-// Register-resident splines shared by the tensor-core forward kernels (flow_tc.cu, flow_tc_h.cu).
+// Register-resident splines of the fp16-split tensor-core kernel (flow_tc_h.cu).
 #pragma once
 #include "spline.cuh"
 
-// PWQuad with 32 bins on a register-resident logit vector z[0..64] (33 vertex heights, 32 widths): the
-// reference's map (coupling_cells.py:167-225, see spline.cuh::pwquad_fwd) with static indexing only — the bin
-// is found by counting edges, the per-bin quantities by predicated accumulation.
-__device__ __forceinline__ void pwquad32_regs(const float* z, float x, float& y, float& f, int& kbin) {
-    float mv = z[0], mw = z[33];
-#pragma unroll
-    for (int j = 1; j <= 32; ++j) mv = fmaxf(mv, z[j]);
-#pragma unroll
-    for (int j = 1; j < 32; ++j) mw = fmaxf(mw, z[33 + j]);
-    float w[32], v[33];
-    double Sw = 0.0;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) { w[j] = expf(z[33 + j] - mw); Sw += (double)w[j]; }
-#pragma unroll
-    for (int j = 0; j <= 32; ++j) v[j] = expf(z[j] - mv);
-    double Araw = 0.0;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) Araw += 0.5 * ((double)v[j] + (double)v[j + 1]) * (double)w[j];
-    const float xb = x > NIS_QUAD_CLAMP ? NIS_QUAD_CLAMP : x;
-    const double target = (double)xb * Sw;
-    int k = 0;
-    double cum = 0.0;
-#pragma unroll
-    for (int j = 0; j < 31; ++j) { cum += (double)w[j]; k += cum <= target ? 1 : 0; }
-    double cw = 0.0, ca = 0.0;
-    float wk = 0.f, vk = 0.f, vk1 = 0.f;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) {
-        const bool below = j < k;
-        cw += below ? (double)w[j] : 0.0;
-        ca += below ? 0.5 * ((double)v[j] + (double)v[j + 1]) * (double)w[j] : 0.0;
-        wk = j == k ? w[j] : wk;
-        vk = j == k ? v[j] : vk;
-        vk1 = j == k ? v[j + 1] : vk1;
-    }
-    const float invA = (float)(Sw / Araw);
-    const float alpha = (float)((target - cw) / (double)wk);
-    const float Vk = vk * invA, Vk1 = vk1 * invA;
-    const float Wk = (float)((double)wk / Sw);
-    y = alpha * alpha * 0.5f * (Vk1 - Vk) * Wk + alpha * Vk * Wk + (float)(ca / Araw);
-    f = Vk + alpha * (Vk1 - Vk);
-    kbin = k;
-}
-
-
-// ---- round 2: the same map with pairwise trees and a binary descent -----------------------------------------------------
-// pwquad32_regs above spends ~920 instructions per transformed dimension, ~400 of them float64 (running sums of the widths
-// and of the trapezoids, 31 float64 compares, two predicated float64 accumulations per bin, four float64 divisions): the
-// PWQuad final pass was 2.0 ms per cell against 0.41 ms for PWLin.  Here only what 1/W_k amplifies stays float64 - the sum
-// of the widths below the bin, from a pairwise tree of float64 partial sums - and the bin is found by descending that tree
-// (5 compares).  The trapezoid sums (no amplification: they enter y and the normalisation directly) are a float32 tree; the
-// per-bin quantities are picked by select trees along the bits of the bin index; the divisions are float32.
-// LOG2: the logits are in units of log 2 (bare ex2).
 __device__ __forceinline__ float tcs_ex2(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -87,7 +34,12 @@ __device__ __forceinline__ T tcs_sel4(const T* a, int st, bool b1, bool b0) {
     return b1 ? hi : lo;
 }
 
-template <bool LOG2>
+// PWQuad with 32 bins on a register-resident logit vector z[0..64] (33 vertex heights, 32 widths, in units of log 2: bare
+// ex2): the reference's map (coupling_cells.py:167-225, see spline.cuh::pwquad_fwd) with pairwise trees and a binary
+// descent.  Only what 1/W_k amplifies stays float64 - the sum of the widths below the bin, from a pairwise tree of float64
+// partial sums - and the bin is found by descending that tree (5 compares).  The trapezoid sums (no amplification: they
+// enter y and the normalisation directly) are a float32 tree; the per-bin quantities are picked by select trees along the
+// bits of the bin index; the divisions are float32.
 __device__ __forceinline__ void pwquad32_tree(const float* z, float x, float& y, float& f, int& kbin) {
     float mv = z[0], mw = z[33];
 #pragma unroll
@@ -96,9 +48,9 @@ __device__ __forceinline__ void pwquad32_tree(const float* z, float x, float& y,
     for (int j = 1; j < 32; ++j) mw = fmaxf(mw, z[33 + j]);
     float w[32], v[33], a[32];
 #pragma unroll
-    for (int j = 0; j < 32; ++j) w[j] = LOG2 ? tcs_ex2(z[33 + j] - mw) : __expf(z[33 + j] - mw);
+    for (int j = 0; j < 32; ++j) w[j] = tcs_ex2(z[33 + j] - mw);
 #pragma unroll
-    for (int j = 0; j <= 32; ++j) v[j] = LOG2 ? tcs_ex2(z[j] - mv) : __expf(z[j] - mv);
+    for (int j = 0; j <= 32; ++j) v[j] = tcs_ex2(z[j] - mv);
 #pragma unroll
     for (int j = 0; j < 32; ++j) a[j] = (v[j] + v[j + 1]) * (0.5f * w[j]);              // trapezoid j (raw widths)
     double W1[16], W2[8], W4[4];
@@ -220,13 +172,12 @@ __device__ __forceinline__ void pwlin32_tree_inv(const float* z, float m, float 
     jinv = S / (32.f * ek);
 }
 
-// PWQuad with 32 bins: y -> x on z[0..64] (33 heights, 32 widths; units of log 2 when LOG2), the inverse of pwquad32_tree.
+// PWQuad with 32 bins: y -> x on z[0..64] (33 heights, 32 widths; units of log 2), the inverse of pwquad32_tree.
 // The bin is found by descending the float32 trapezoid-area tree with target y A_raw (the largest k with S_k <= y, as
 // spline.cuh::pwquad_inv); E_k Sw is picked from the float64 width tree along the same bits.  Inside the bin
 // y - S_k = alpha V_k W_k + alpha^2 (V_{k+1} - V_k) W_k / 2, scaled by A_raw: c = target - A_k, b = v_k w_k,
 // a = (v_{k+1} - v_k) w_k / 2, alpha = 2c / (b + sqrt(b^2 + 4ac)) (no cancellation for a < 0).  x = (E_k Sw + alpha w_k) / Sw,
 // jinv = 1 / f with f = V_k + alpha (V_{k+1} - V_k).  The forward reads x only up to NIS_QUAD_CLAMP, so x is clamped there.
-template <bool LOG2>
 __device__ __forceinline__ void pwquad32_tree_inv(const float* z, float y, float& x, float& jinv, int& kbin) {
     float mv = z[0], mw = z[33];
 #pragma unroll
@@ -235,9 +186,9 @@ __device__ __forceinline__ void pwquad32_tree_inv(const float* z, float y, float
     for (int j = 1; j < 32; ++j) mw = fmaxf(mw, z[33 + j]);
     float w[32], v[33], a[32];
 #pragma unroll
-    for (int j = 0; j < 32; ++j) w[j] = LOG2 ? tcs_ex2(z[33 + j] - mw) : __expf(z[33 + j] - mw);
+    for (int j = 0; j < 32; ++j) w[j] = tcs_ex2(z[33 + j] - mw);
 #pragma unroll
-    for (int j = 0; j <= 32; ++j) v[j] = LOG2 ? tcs_ex2(z[j] - mv) : __expf(z[j] - mv);
+    for (int j = 0; j <= 32; ++j) v[j] = tcs_ex2(z[j] - mv);
 #pragma unroll
     for (int j = 0; j < 32; ++j) a[j] = (v[j] + v[j + 1]) * (0.5f * w[j]);
     double W1[16], W2[8], W4[4];

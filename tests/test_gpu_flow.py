@@ -107,27 +107,32 @@ def test_bench_configuration_against_the_oracle_at_a_million_points(mode):
     test_forward_matches_oracle_at_size(dict(BIG[0], B=1 << 20), mode, max_log_j=1e-4)
 
 
-@pytest.mark.parametrize("backend", ["tcgen05", "tcgen05_3xtf32", "fp32_tiled_4x8", "fp32_tiled_8x8", "generic"])
+# cfg2, cfg4, cfg5_small, and two width-64 flows whose fp16-split launch sequences differ from cfg2's and cfg4's: PWLin at
+# depth 2 with six pass-through columns (no recomputed last layer, column moments in a launch of their own for every cell),
+# and PWQuad with one hidden layer (the final pass starts from the state)
+FAMILY = [BIG[0], BIG[1], BIG[3],
+          dict(name="lin8d_depth2_6pass", kind="lin", n_flow=8, n_pass_through=6, n_cells=4, n_bins=32, NN=[64] * 2,
+               roll_step=3, B=1 << 13),
+          dict(name="quad8d_1layer", kind="quad", n_flow=8, n_cells=4, n_bins=32, NN=[64], B=1 << 13)]
+
+
+@pytest.mark.parametrize("backend", ["tcgen05", "fp32_tiled_4x8", "generic"])
 @pytest.mark.parametrize("mode", ["eval", "train"])
-@pytest.mark.parametrize("which", [0, 1, 3], ids=["cfg2", "cfg4", "cfg5_small"])
-def test_every_kernel_family_agrees_with_the_oracle(monkeypatch, backend, mode, which):
-    """cfg2 (PWLin) and cfg4 (PWQuad) are served by the resident-weights tcgen05 kernel by default, the 256-wide
-    cfg5 by the streamed-weights one (flow_wide.cu); the FP32-pipe register-tiled kernels and the shape-generic
-    kernel stay selectable (library test knobs) and must meet the same parity bar."""
-    if which == 3 and backend.startswith("fp32_tiled"):
+@pytest.mark.parametrize("cfg", FAMILY, ids=[c["name"] for c in FAMILY])
+def test_every_kernel_family_agrees_with_the_oracle(monkeypatch, backend, mode, cfg):
+    """The width-64 flows with 32 bins are served by the fp16-split tcgen05 kernel by default, the 256-wide cfg5 by the
+    streamed-weights one (flow_wide.cu); the FP32-pipe register-tiled kernel and the shape-generic kernel stay
+    selectable (library test knobs) and must meet the same parity bar."""
+    if cfg["NN"][0] != 64 and backend.startswith("fp32_tiled"):
         pytest.skip("the register-tiled FP32 kernels are width-64 only")
-    if backend == "tcgen05_3xtf32" and which != 0:
-        pytest.skip("only the PWLin width-64 cells have two tensor-core kernels (fp16-split default, 3xTF32 with NIS_TC_H=0)")
-    env = {"tcgen05": {}, "tcgen05_3xtf32": {"NIS_TC_H": "0"}, "fp32_tiled_4x8": {"NIS_TC": "0"}, "fp32_tiled_8x8": {"NIS_TC": "0", "NIS_TILED_VARIANT": "8"},
-           "generic": {"NIS_TC": "0", "NIS_DISABLE_TILED": "1"}}[backend]
-    for k in ("NIS_TC", "NIS_TC_H", "NIS_TILED_VARIANT", "NIS_DISABLE_TILED"):
+    env = {"tcgen05": {}, "fp32_tiled_4x8": {"NIS_TC": "0"}, "generic": {"NIS_TC": "0", "NIS_DISABLE_TILED": "1"}}[backend]
+    for k in ("NIS_TC", "NIS_DISABLE_TILED"):
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    test_forward_matches_oracle_at_size(BIG[which], mode)
-    # ragged batch (not a multiple of any tile size) through the same kernels
-    cfg = dict(BIG[which], B=(1 << 13) + 77)
     test_forward_matches_oracle_at_size(cfg, mode)
+    # ragged batch (not a multiple of any tile size) through the same kernels
+    test_forward_matches_oracle_at_size(dict(cfg, B=(1 << 13) + 77), mode)
 
 
 def test_flow_is_a_bijection_of_the_unit_cube_at_full_size():

@@ -133,8 +133,7 @@ def test_tensor_core_and_generic_inverses_match_the_oracle(monkeypatch, cfg, mod
     NF, model, sd = _model(cfg, mode)
     yj = _points(cfg)
     ref = Oracle(cfg, mode, sd, yj)
-    for k in ("NIS_TC", "NIS_TC_H"):
-        monkeypatch.delenv(k, raising=False)
+    monkeypatch.delenv("NIS_TC", raising=False)
     tags = launch_tags(lambda: model.spec().inverse(yj.cuda(), model.training, want_bins=True))
     assert sum(t >= 10 for t in tags) >= cfg["n_cells"], tags
     X, bins = model.spec().inverse(yj.cuda(), model.training, want_bins=True)
@@ -220,8 +219,7 @@ def test_train_mode_inverse_leaves_the_running_statistics_alone():
 def test_dispatch(monkeypatch, mode):
     """A supported shape at B >= 256 runs the tensor-core cell kernel (tags 10 .. 13); NIS_TC=0 and a shape outside it
     (6 bins, width 16) run only the shape-generic kernel (tag 2, after the weight pack, tag 0)."""
-    for k in ("NIS_TC", "NIS_TC_H"):
-        monkeypatch.delenv(k, raising=False)
+    monkeypatch.delenv("NIS_TC", raising=False)
     cfg = dict(CFG2, B=4096)
     NF, model, _ = _model(cfg, mode)
     yj = _points(cfg).cuda()

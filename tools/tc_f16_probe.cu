@@ -1,4 +1,4 @@
-// Probe for the fp16-split conditioner path (flow_tc.cu, round 2):
+// Probe for the fp16-split conditioner path (flow_tc_h.cu, round 2):
 //   (1) layout check: tcgen05.mma.kind::f16 with the A operand in TENSOR MEMORY as packed half2 (column c of lane m
 //       holds K elements 2c (low half) and 2c+1 (high half)), B in shared memory K-major / 128-byte swizzle,
 //       fp32 accumulator — compared with a host product;

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Times the cfg2 flow forward (eval and train BN) on 2^22 points with CUDA events; honours the tuning
-environment knobs of the library (NIS_DISABLE_TILED, NIS_TILED_VARIANT).  Development aid."""
+environment knobs of the library (NIS_TC, NIS_DISABLE_TILED).  Development aid."""
 import os
 import sys
 
@@ -30,6 +30,6 @@ for mode in ("eval", "train"):
         e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 5
-    print(kind + " %s variant=%s mode=%s: %.3f ms  %.3e pts/s  %.1f TFLOP/s algorithmic" % (
-        os.environ.get("NIS_DISABLE_TILED", "0"), os.environ.get("NIS_TILED_VARIANT", "8"), mode, ms, n / ms * 1e3,
+    print(kind + " NIS_TC=%s NIS_DISABLE_TILED=%s mode=%s: %.3f ms  %.3e pts/s  %.1f TFLOP/s algorithmic" % (
+        os.environ.get("NIS_TC", "1"), os.environ.get("NIS_DISABLE_TILED", "0"), mode, ms, n / ms * 1e3,
         n * 199680 / ms / 1e9))
