@@ -23,7 +23,7 @@
  * unless marked host; work is enqueued on `stream` and the call returns without synchronising; no
  * allocation; re-entrant.  Process-wide state is limited to caches of launch attributes (the dynamic
  * shared-memory opt-in per kernel and device, the SM count) and to environment variables that select a
- * kernel family for tests and A/B measurements (NIS_TC, NIS_DISABLE_TILED, NIS_BWD_TC, ... - INTEGRATION.md section 7;
+ * kernel family for tests and A/B measurements (NIS_TC, NIS_DISABLE_TILED, NIS_BWD_TC - INTEGRATION.md section 7;
  * read on every call, unset in production); the measurement aid nis_flow_timing_* keeps a per-thread
  * event list.  Return value: 0 on success, a negative NIS_E* code otherwise (nis_strerror() gives
  * text).  `stream` is a cudaStream_t passed as void*.

@@ -25,6 +25,17 @@
         }                                                                                                 \
     } while (0)
 
+// Streaming multiprocessors of the current device, queried once per device (148, a B200's count, if the query fails).
+static inline int nis_sm_count() {
+    static int sms[16] = {0};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    dev &= 15;
+    if (sms[dev] <= 0 && (cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms[dev] <= 0))
+        sms[dev] = 148;
+    return sms[dev];
+}
+
 static inline __host__ __device__ int pad8(int x) { return (x + 7) & ~7; }
 static inline __host__ __device__ int pad4(int x) { return (x + 3) & ~3; }
 

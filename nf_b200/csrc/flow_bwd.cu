@@ -21,6 +21,7 @@
 #include <cooperative_groups.h>
 #include "common.cuh"
 #include "spline.cuh"
+#include "flow_host.cuh"
 
 // floats between the BN-backward means of consecutive layers: whole 128-byte lines per layer (a layer's block is rewritten by
 // one CTA of the cooperative kernel while the others may hold its neighbours in L1)
@@ -556,22 +557,6 @@ static int launch_bwd(const DevFlow& F, const BwdArgs& A, int grid, cudaStream_t
     return NIS_OK;
 }
 
-__global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_running,
-                                 float* __restrict__ wpack, int bn_mode);
-
-// tensor-core train-mode backward (flow_bwd_tc.cu)
-bool nis_bwd_tc_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                         const float* saved, const float* bn_saved, const void* grad_out, int grad_dtype,
-                         float* grad_params, void* grad_in, int64_t B, cudaStream_t s);
-
-// wide-conditioner train-mode backward (flow_bwd_wide.cu)
-bool nis_bwd_wide_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                           const float* saved, const float* bn_saved, const float* act_saved, const void* grad_out, int grad_dtype,
-                           float* grad_params, void* grad_in, int64_t B, cudaStream_t s);
-size_t nis_act_cache_floats(const DevFlow& F, int64_t B);
-
 static int launch_bwd_any(const DevFlow& F, const BwdArgs& A, int NT, int grid, cudaStream_t s) {
     switch (NT) {
         case 128: return launch_bwd<128>(F, A, grid, s);
@@ -606,11 +591,12 @@ extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* pa
     cudaStream_t s = (cudaStream_t)stream;
     FlowWorkspace ws;
     nis_flow_carve(F, B, workspace, &ws);
-    if (nis_bwd_tc_supported(F, B, bn_mode))
+    const FlowPlan plan = nis_flow_plan(F, B, bn_mode);
+    if (plan.bwd == BWD_TC)
         return nis_flow_backward_tc(F, ws, params, bn_running, saved, bn_saved, grad_out, grad_dtype, grad_params, grad_in, B, s);
-    if (nis_bwd_wide_supported(F, B, bn_mode))
-        return nis_flow_backward_wide(F, ws, params, bn_running, saved, bn_saved,
-                                      nis_act_cache_floats(F, B) ? act_saved : nullptr, grad_out, grad_dtype, grad_params, grad_in, B, s);
+    if (plan.bwd == BWD_WIDE)
+        return nis_flow_backward_wide(F, ws, params, bn_running, saved, bn_saved, plan.act_cache ? act_saved : nullptr,
+                                      grad_out, grad_dtype, grad_params, grad_in, B, s);
     bool rotate = false;
     const int NT = bwd_pick_nt(F, train != 0, &rotate);
     if (!NT) return NIS_EUNSUPPORTED;
@@ -618,19 +604,10 @@ extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* pa
     bwd_carve(F, B, ws.bwd, &sc);
     const int grid = bwd_grid(F, B, NT);
     cudaMemsetAsync(ws.counter, 0, 256, s);
-    {
-        int mx = 0;
-        for (int c = 0; c < F.n_cells; ++c) {
-            int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
-            if (sz > mx) mx = sz;
-        }
-        int bx = (mx + 255) / 256;
-        if (bx > 64) bx = 64;
-        flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, bn_mode);
-        NIS_CUDA_CHECK_LAUNCH();
-        flow_bwd_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, sc.wb, bn_saved, ws.wpack, train);
-        NIS_CUDA_CHECK_LAUNCH();
-    }
+    rc = launch_flow_pack(F, params, bn_running, ws.wpack, bn_mode, s);
+    if (rc) return rc;
+    flow_bwd_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, sc.wb, bn_saved, ws.wpack, train);
+    NIS_CUDA_CHECK_LAUNCH();
     BwdArgs A;
     A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype;
     A.gstate = sc.gstate; A.dact = sc.dact; A.params = params; A.wpack = ws.wpack; A.wb = sc.wb;
@@ -639,21 +616,19 @@ extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* pa
     const int OUT = F.depth + 1;
     if (train && NT == 128 && !rotate) {
         // small batch: the whole backward in one cooperative launch when every tile has its own resident CTA
-        static const int coop_env = [] { const char* e = getenv("NIS_COOP"); return e && e[0] == '0' ? 0 : 1; }();
         const long long ntiles = (B + NT - 1) / NT;
         const size_t smem = bwd_smem_bytes(F, 128, false);
         static int maxg[16] = {0};
         int dev = 0;
         cudaGetDevice(&dev);
         dev &= 15;
-        if (coop_env && maxg[dev] == 0) {
-            int per_sm = 0, sms = 0;
+        if (maxg[dev] == 0) {
+            int per_sm = 0;
             NIS_ENSURE_SMEM((flow_bwd_coop_kernel<128>), (int)smem);
             cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, flow_bwd_coop_kernel<128>, 128, smem);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            maxg[dev] = per_sm * sms > 0 ? per_sm * sms : -1;
+            maxg[dev] = per_sm > 0 ? per_sm * nis_sm_count() : -1;
         }
-        if (coop_env && ntiles == grid && ntiles <= maxg[dev]) {
+        if (ntiles == grid && ntiles <= maxg[dev]) {
             NIS_ENSURE_SMEM((flow_bwd_coop_kernel<128>), (int)smem);
             A.grad_in = grad_in; A.c = 0; A.cell_params = 0; A.first = 1; A.step_begin = A.step_end = OUT;
             void* args[] = {(void*)&F, (void*)&A};

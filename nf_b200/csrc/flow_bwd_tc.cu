@@ -28,6 +28,7 @@
 #include <stdlib.h>
 #include "common.cuh"
 #include "tc_common.cuh"
+#include "flow_host.cuh"
 
 #define BT_GROUP_COLS 192     // per point group: dz hi [0,64), dz lo [64,128), dgrad accumulator [128,192)
 #define BT_COL_LO 64
@@ -876,16 +877,11 @@ int nis_tc_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream
     return NIS_OK;
 }
 
-int64_t nis_tc_min_batch(int64_t dflt);
-
 // Width-64 cells with 32 bins (PWLin or PWQuad) whose operands in the 3xTF32 layout (tc_layout) fit an SM's shared memory
 // in each launch shape of the round-1 forward: fused eval cell, layer pass, final pass.  The tensor-core backward below
-// takes the PWLin ones; flow_fwd.cu runs the fp16-split forward and inverse only on shapes this accepts.
-bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode) {
-    (void)bn_mode;
-    const char* off = getenv("NIS_TC");                   // NIS_TC=0 forces the FP32-pipe kernels (test knob)
-    if (off && off[0] == '0') return false;
-    if (F.depth < 1 || B < nis_tc_min_batch(256) || F.maxW != TCH || F.nb != 32) return false;
+// takes the PWLin ones; the fp16-split forward and inverse take all of them (nis_flow_plan).
+bool nis_tc_supported(const DevFlow& F) {
+    if (F.depth < 1 || F.maxW != TCH || F.nb != 32) return false;
     for (int l = 0; l < F.depth; ++l) if (F.widths[l] != TCH) return false;
     if (F.kind == NIS_KIND_PWLIN ? F.K != 32 : F.K != 65) return false;
     for (int c = 0; c < F.n_cells; ++c) {
@@ -900,24 +896,10 @@ bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode) {
     return true;
 }
 
-__global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_running,
-                                 float* __restrict__ wpack, int bn_mode);
-
-bool nis_bwd_tc_supported(const DevFlow& F, int64_t B, int bn_mode) {
-    const char* off = getenv("NIS_BWD_TC");               // NIS_BWD_TC=0 forces the shape-generic backward (test knob)
-    if (off && off[0] == '0') return false;
-    if (bn_mode != NIS_BN_TRAIN || F.kind != NIS_KIND_PWLIN || F.K != 32) return false;
-    if (!nis_tc_supported(F, B, bn_mode)) return false;
-    for (int c = 0; c < F.n_cells; ++c)
-        if (F.cells[c].P > 16 || F.cells[c].T * F.K > TC_NOUT) return false;
-    return true;
-}
+bool nis_bwd_tc_supported(const DevFlow& F) { return F.kind == NIS_KIND_PWLIN && nis_tc_supported(F); }
 
 static int bt_grid(int64_t B) {
-    int sms = 0, dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
+    const int sms = nis_sm_count();
     const long long npairs = ((B + TCM - 1) / TCM + 1) / 2;
     return (int)(npairs < sms ? npairs : sms);
 }
@@ -952,39 +934,23 @@ int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float*
     int grid = bt_grid(B);
     if (grid > 148) grid = 148;
     cudaMemsetAsync(ws.counter, 0, 256, s);
-    {
-        int mx = 0;
-        for (int c = 0; c < F.n_cells; ++c) {
-            int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
-            if (sz > mx) mx = sz;
-        }
-        int bx = (mx + 255) / 256;
-        if (bx > 64) bx = 64;
-        flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, NIS_BN_TRAIN);
-        NIS_CUDA_CHECK_LAUNCH();
-        flow_bwd_tc_pack_kernel<<<dim3(16, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.bdpack);
-        NIS_CUDA_CHECK_LAUNCH();
-        int rc = nis_tc_pack(F, params, ws.tcpack, s);
-        if (rc) return rc;
-    }
+    int rc = launch_flow_pack(F, params, bn_running, ws.wpack, NIS_BN_TRAIN, s);
+    if (rc) return rc;
+    flow_bwd_tc_pack_kernel<<<dim3(16, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.bdpack);
+    NIS_CUDA_CHECK_LAUNCH();
+    rc = nis_tc_pack(F, params, ws.tcpack, s);
+    if (rc) return rc;
     BtArgs A;
     A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype; A.grad_in = nullptr;
     A.gstate = sc.gstate; A.params = params; A.wpack = ws.wpack; A.bn_saved = bn_saved;
     A.tcpack = ws.tcpack; A.bdpack = sc.bdpack; A.zbuf = sc.zbuf; A.dl = sc.dl;
     A.bnb = sc.bnb; A.slices = sc.slices; A.grad_params = grad_params;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B; A.ntiles = (B + TCM - 1) / TCM; A.grid = grid;
-    A.dh_in = nullptr; A.dh_out = nullptr; A.lam = 0;
-    {
-        const char* fe = getenv("NIS_BWD_FLUSH");         // test knob: 0 = accumulate over the whole CTA without flushing
-        A.flush_every = fe ? atoi(fe) : BT_FLUSH;
-    }
+    A.dh_in = nullptr; A.dh_out = nullptr; A.lam = 0; A.flush_every = BT_FLUSH;
     const size_t smem64 = (size_t)bt_layout(64).total + 1024, smem128 = (size_t)bt_layout(128).total + 1024;
     NIS_ENSURE_SMEM((flow_bwd_tc_layer_kernel<64>), (int)smem64);
     NIS_ENSURE_SMEM((flow_bwd_tc_layer_kernel<128>), (int)smem128);
-    int sms1 = 0, dev1 = 0;
-    cudaGetDevice(&dev1);
-    cudaDeviceGetAttribute(&sms1, cudaDevAttrMultiProcessorCount, dev1);
-    if (sms1 <= 0) sms1 = 148;
+    const int sms1 = nis_sm_count();
     const long long nt1 = (B + TCM - 1) / TCM;
     const int grid1 = (int)(nt1 < sms1 ? nt1 : sms1);
     const int lgrid = grid1;                               // CTAs of the layer launches (one tile at a time each) = slices per layer

@@ -26,6 +26,7 @@
 #include "tc_common.cuh"
 #include "wide_common.cuh"
 #include "flow_fwd_common.cuh"
+#include "flow_host.cuh"
 
 struct BwArgs {
     const float* saved; const void* grad_out; int grad_dtype;
@@ -942,16 +943,8 @@ __global__ void __launch_bounds__(256) flow_bwd_wide_tail_kernel(const __grid_co
 }
 
 // ---------------------------------------------------------------------------------------------------
-bool nis_wide_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_wide_pack(const DevFlow& F, const float* params, float* widepack, cudaStream_t s);
-int nis_launch_wide(const DevFlow& F, const FwdArgs& A, const float* widepack, cudaStream_t s);
-__global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_running,
-                                 float* __restrict__ wpack, int bn_mode);
-
-bool nis_bwd_wide_supported(const DevFlow& F, int64_t B, int bn_mode) {
-    const char* off = getenv("NIS_BWD_TC");               // NIS_BWD_TC=0 forces the shape-generic backward (test knob)
-    if (off && off[0] == '0') return false;
-    if (bn_mode != NIS_BN_TRAIN || !nis_wide_supported(F, B, bn_mode)) return false;
+bool nis_bwd_wide_supported(const DevFlow& F) {
+    if (!nis_wide_supported(F, NIS_BN_TRAIN)) return false;
     const int W = F.widths[0];
     if (W != 64 && W != 128 && W != 256) return false;      // wgrad column blocks of min(W, 128)
     for (int c = 0; c < F.n_cells; ++c) {
@@ -990,29 +983,17 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
                            float* grad_params, void* grad_in, int64_t B, cudaStream_t s) {
     BwScratch sc;
     bw_carve(F, B, ws.bwd, &sc);
-    int sms = 0, dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
+    const int sms = nis_sm_count();
     const long long ntiles = (B + TCM - 1) / TCM;
     const int grid = (int)(ntiles < sms ? ntiles : sms);
     const int W = F.widths[0], Kp = wd_kp16(F), depth = F.depth;
     cudaMemsetAsync(ws.counter, 0, 256, s);
-    {
-        int mx = 0;
-        for (int c = 0; c < F.n_cells; ++c) {
-            int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
-            if (sz > mx) mx = sz;
-        }
-        int bx = (mx + 255) / 256;
-        if (bx > 64) bx = 64;
-        flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, NIS_BN_TRAIN);
-        NIS_CUDA_CHECK_LAUNCH();
-        flow_bwd_wide_pack_kernel<<<dim3(128, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.dgpack);
-        NIS_CUDA_CHECK_LAUNCH();
-        int rc = nis_wide_pack(F, params, ws.tcpack, s);
-        if (rc) return rc;
-    }
+    int rc = launch_flow_pack(F, params, bn_running, ws.wpack, NIS_BN_TRAIN, s);
+    if (rc) return rc;
+    flow_bwd_wide_pack_kernel<<<dim3(128, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.dgpack);
+    NIS_CUDA_CHECK_LAUNCH();
+    rc = nis_wide_pack(F, params, ws.tcpack, s);
+    if (rc) return rc;
     BwArgs A;
     A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype; A.gstate = sc.gstate;
     A.params = params; A.wpack = ws.wpack; A.bn_saved = bn_saved; A.widepack = ws.tcpack; A.dgpack = sc.dgpack;
@@ -1033,18 +1014,17 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
             A.zbuf = act_saved + (size_t)c * depth * ntiles * tile_fl;
         } else {
             FwdArgs Fa;
-            Fa.in = nullptr; Fa.in_dtype = NIS_F32; Fa.in_cols = F.d + 1;
-            Fa.state_in = saved + (long long)c * rows; Fa.state_out = nullptr; Fa.out = nullptr; Fa.out_dtype = NIS_F32;
-            Fa.from_state = 1; Fa.to_out = 0; Fa.saved = nullptr; Fa.bins = nullptr;
-            Fa.params = params; Fa.wpack = ws.wpack; Fa.bn_running = nullptr; Fa.bn_saved = nullptr;
-            Fa.partials = ws.partials; Fa.counter = ws.counter; Fa.B = B; Fa.c_begin = c; Fa.c_end = c + 1;
+            Fa.in_cols = F.d + 1;
+            Fa.state_in = saved + (long long)c * rows; Fa.from_state = 1;
+            Fa.params = params; Fa.wpack = ws.wpack; Fa.partials = ws.partials; Fa.counter = ws.counter;
+            Fa.B = B; Fa.c_begin = c; Fa.c_end = c + 1;
             Fa.no_stats = 1;
             for (int l = 2; l <= depth; ++l) {
                 Fa.stats_layer = l;
                 Fa.zin = l > 2 ? sc.zbuf + (size_t)(l - 2) * ntiles * tile_fl : nullptr;
                 Fa.zout = sc.zbuf + (size_t)(l - 1) * ntiles * tile_fl;
                 Fa.z1out = l == 2 ? sc.zbuf : nullptr;
-                int rc = nis_launch_wide(F, Fa, ws.tcpack, s);
+                rc = nis_launch_wide(F, Fa, ws.tcpack, s);
                 if (rc) return rc;
             }
         }

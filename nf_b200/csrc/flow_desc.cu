@@ -1,6 +1,8 @@
-// Host-side descriptor handling for the flow kernels: validation, arena layouts, workspace carve-up.
+// Host-side descriptor handling for the flow kernels: validation, arena layouts, workspace carve-up, kernel plan.
+#include <stdlib.h>
 #include <string.h>
 #include "common.cuh"
+#include "flow_host.cuh"
 
 static int cond_out(const NisFlowDesc* d) {
     return d->kind == NIS_KIND_PWLIN ? d->n_bins : (d->kind == NIS_KIND_AFFINE ? 2 : 2 * d->n_bins + 1);
@@ -90,11 +92,39 @@ extern "C" int64_t nis_flow_bn_saved_count(const NisFlowDesc* d) {
 
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
+// Smallest batches the tensor-core kernels (fp16-split, streamed-weights, both tensor-core backwards) and the register-
+// tiled kernel take; smaller ones run on the kernels of the next family down.
+static const int64_t TC_MIN_BATCH = 256;
+static const int64_t TILED_MIN_BATCH = 2048;
+
+// Which kernel family runs one call.  Knobs, read on every call so that a process can switch between them (the tests
+// compare each family against the reference kernels this way): NIS_TC=0 disables the tensor-core forwards and backwards,
+// NIS_DISABLE_TILED=1 the register-tiled forward, NIS_BWD_TC=0 both tensor-core backwards.
+// The fp16-split forward and inverse take the shapes nis_tc_supported accepts.  Its own shared-memory limit (at least two
+// point groups per CTA) is met by each of them: a sweep of the 6256 width-64, 32-bin PWLin and PWQuad shapes with n_flow
+// 2-32, P 1-17 and depth 1-8 found none it rejects.  It would accept about five times as many shapes (for example every
+// n_flow >= 10 at depth 1), which run on the streamed-weights kernel; giving them to the fp16-split kernel needs parity
+// tests and B200 timings against that kernel of their own.
+FlowPlan nis_flow_plan(const DevFlow& F, int64_t B, int bn_mode) {
+    auto knob = [](const char* name, char value) { const char* e = getenv(name); return e && e[0] == value; };
+    const bool tc = B >= TC_MIN_BATCH && !knob("NIS_TC", '0');
+    const bool train = bn_mode == NIS_BN_TRAIN;
+    FlowPlan p;
+    if (tc && nis_tc_supported(F)) p.fwd = FWD_H;
+    else if (tc && nis_wide_supported(F, bn_mode)) p.fwd = FWD_WIDE;
+    else if (B >= TILED_MIN_BATCH && !knob("NIS_DISABLE_TILED", '1') && nis_tiled_supported(F)) p.fwd = FWD_TILED;
+    else p.fwd = FWD_GENERIC;
+    const bool bwd_tc = train && tc && !knob("NIS_BWD_TC", '0');
+    if (bwd_tc && nis_bwd_tc_supported(F)) p.bwd = BWD_TC;
+    else if (bwd_tc && nis_bwd_wide_supported(F)) p.bwd = BWD_WIDE;
+    else p.bwd = BWD_GENERIC;
+    // both sides on the wide kernels: the backward can skip the layer passes
+    p.act_cache = p.fwd == FWD_WIDE && p.bwd == BWD_WIDE && F.depth >= 2;
+    return p;
+}
+
 // Backward scratch (floats), see flow_bwd.cu: gradient state [B][d+1], per-CTA parameter-gradient
 // partials [NIS_BWD_GRID][max cell params], BN backward sums [n_cells][depth+1][2][maxW].
-
-size_t nis_tc_pack_floats(const DevFlow& F);
-size_t nis_wide_pack_floats(const DevFlow& F);
 
 size_t nis_flow_carve(const DevFlow& F, int64_t B, void* base, FlowWorkspace* ws) {
     size_t off = 0;

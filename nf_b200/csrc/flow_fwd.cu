@@ -16,6 +16,7 @@
 #include "spline.cuh"
 #include <cooperative_groups.h>
 #include "flow_fwd_common.cuh"
+#include "flow_host.cuh"
 
 // ---------------------------------------------------------------------------------------------------
 // repack: torch-layout params -> transposed zero-padded weights (+ eval-mode BN scale/shift)
@@ -66,6 +67,23 @@ __global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, co
         const int t = i / Kp, j = i - t * Kp;
         pk[q.bo_off + i] = j < K ? bo[F.out_row(c, t, j)] : 0.f;
     }
+}
+
+// one block per 256 floats of the largest cell, at most 64
+int nis_pack_blocks(const DevFlow& F) {
+    int mx = 0;
+    for (int c = 0; c < F.n_cells; ++c) {
+        int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
+        if (sz > mx) mx = sz;
+    }
+    int bx = (mx + 255) / 256;
+    return bx > 64 ? 64 : bx;
+}
+
+int launch_flow_pack(const DevFlow& F, const float* params, const float* bn_running, float* wpack, int bn_mode, cudaStream_t s) {
+    flow_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, bn_running, wpack, bn_mode);
+    NIS_CUDA_CHECK_LAUNCH();
+    return NIS_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -281,27 +299,6 @@ __global__ void __launch_bounds__(NT) flow_fwd_coop_kernel(const __grid_constant
 // ---------------------------------------------------------------------------------------------------
 // launcher
 // ---------------------------------------------------------------------------------------------------
-size_t nis_flow_bwd_scratch_floats(const DevFlow& F, int64_t B);
-bool nis_tiled_supported(const DevFlow& F, int64_t B);
-size_t nis_tiled_zbuf_floats(int64_t B);
-bool nis_tc_supported(const DevFlow& F, int64_t B, int bn_mode);
-bool nis_h_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_h_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s);
-int nis_launch_h(const DevFlow& F, const FwdArgs& A, const float* tcpack, cudaStream_t s);
-bool nis_bwd_tc_supported(const DevFlow& F, int64_t B, int bn_mode);
-bool nis_wide_supported(const DevFlow& F, int64_t B, int bn_mode);
-int nis_wide_pack(const DevFlow& F, const float* params, float* widepack, cudaStream_t s);
-int nis_launch_wide(const DevFlow& F, const FwdArgs& A, const float* widepack, cudaStream_t s);
-// floats of one stored-activation buffer ([tile][width][128], tiles padded to pairs)
-static size_t zbuf_floats(const DevFlow& F, int64_t B) { return nis_tiled_zbuf_floats(B) / 64 * (size_t)(F.maxW > 64 ? F.maxW : 64); }
-size_t nis_bwd_tc_scratch_floats(const DevFlow& F, int64_t B);
-bool nis_bwd_wide_supported(const DevFlow& F, int64_t B, int bn_mode);
-size_t nis_bwd_wide_scratch_floats(const DevFlow& F, int64_t B);
-int nis_launch_tiled(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
-int nis_launch_col_stats(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
-bool nis_moments_supported(const DevFlow& F, int c);
-int nis_launch_col_moments(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
-
 // ---- measurement aid: per-launch device times of nis_flow_forward and nis_flow_inverse (bench.py's roofline object) -----
 // nis_flow_timing_begin() arms a per-thread sink; every kernel launch of the following nis_flow_forward / nis_flow_inverse
 // calls is then bracketed by CUDA events recorded on the launch stream; nis_flow_timing_end() synchronises those events and
@@ -347,19 +344,24 @@ static size_t fwd_smem_bytes(const DevFlow& F, int NT) {
     return fl * sizeof(float) + sizeof(double) * 2 * F.maxW;
 }
 
+// floats of one stored-activation buffer ([tile][width][128], tiles padded to pairs)
+static size_t zbuf_floats(const DevFlow& F, int64_t B) { return nis_tiled_zbuf_floats(B) / 64 * (size_t)(F.maxW > 64 ? F.maxW : 64); }
+
 extern "C" size_t nis_flow_workspace_bytes(const NisFlowDesc* desc, int64_t B) {
     DevFlow F;
     if (nis_build_dev_flow(desc, &F) != NIS_OK || B < 0) return 0;
     FlowWorkspace ws;
     size_t fwd = nis_flow_carve(F, B, nullptr, &ws);
-    // the backward scratch and the tiled train path's activation buffers are never live together
+    // one workspace serves both BN modes: what the train-mode and the eval-mode plan need.  The backward scratch and the
+    // forward's activation buffers are never live together.
+    const FlowPlan train = nis_flow_plan(F, B, NIS_BN_TRAIN), eval = nis_flow_plan(F, B, NIS_BN_EVAL);
     size_t tail = nis_flow_bwd_scratch_floats(F, B);
-    const size_t zfl = (nis_tiled_supported(F, B) || nis_tc_supported(F, B, NIS_BN_TRAIN) || nis_wide_supported(F, B, NIS_BN_EVAL))
-                           ? 2 * zbuf_floats(F, B) : 0;
+    const size_t zfl = (train.fwd != FWD_GENERIC || eval.fwd != FWD_GENERIC) ? 2 * zbuf_floats(F, B) : 0;
     if (zfl > tail) tail = zfl;
-    const size_t tcb = nis_bwd_tc_supported(F, B, NIS_BN_TRAIN) ? nis_bwd_tc_scratch_floats(F, B) : 0;
+    const size_t tcb = train.bwd == BWD_TC ? nis_bwd_tc_scratch_floats(F, B) : 0;
     if (tcb > tail) tail = tcb;
-    const size_t wdb = nis_bwd_wide_supported(F, B, NIS_BN_TRAIN) ? nis_bwd_wide_scratch_floats(F, B) : 0;
+    // (the wide backward's scratch is also reserved where the tensor-core backward takes the shape first)
+    const size_t wdb = (train.bwd != BWD_GENERIC && nis_bwd_wide_supported(F)) ? nis_bwd_wide_scratch_floats(F, B) : 0;
     if (wdb > tail) tail = wdb;
     return fwd + sizeof(float) * tail + 256;
 }
@@ -384,11 +386,10 @@ static int coop_max_grid(size_t smem) {
     cudaGetDevice(&dev);
     dev &= 15;
     if (cached[dev] == 0 || cached_smem[dev] != smem) {
-        int per_sm = 0, sms = 0;
+        int per_sm = 0;
         NIS_ENSURE_SMEM((flow_fwd_coop_kernel<NT>), (int)smem);
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, flow_fwd_coop_kernel<NT>, NT, smem);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        cached[dev] = per_sm * sms > 0 ? per_sm * sms : -1;
+        cached[dev] = per_sm > 0 ? per_sm * nis_sm_count() : -1;
         cached_smem[dev] = smem;
     }
     return cached[dev];
@@ -421,25 +422,12 @@ static int launch_fwd_any(const DevFlow& F, const FwdArgs& A, cudaStream_t s) {
 // Activation cache of the streamed-weights path (cfg5-like shapes): a train-mode forward that a backward will follow can
 // keep z_1..z_depth of every cell ([cell][layer][tile][W][128] float32) so that the backward does not run the layer passes
 // again.  Nonzero only where both the forward and the backward take the wide kernels.
-size_t nis_act_cache_floats(const DevFlow& F, int64_t B) {
-    if (B <= 0 || F.depth < 2) return 0;
-    if (nis_tc_supported(F, B, NIS_BN_TRAIN) || !nis_wide_supported(F, B, NIS_BN_TRAIN)) return 0;
-    if (nis_bwd_tc_supported(F, B, NIS_BN_TRAIN) || !nis_bwd_wide_supported(F, B, NIS_BN_TRAIN)) return 0;
-    const size_t tiles = (size_t)((B + 127) / 128);
-    return (size_t)F.n_cells * F.depth * tiles * F.widths[0] * 128;
-}
-
 extern "C" int64_t nis_flow_act_saved_count(const NisFlowDesc* desc, int64_t B) {
     DevFlow F;
-    if (nis_build_dev_flow(desc, &F) != NIS_OK || B < 0) return 0;
-    return (int64_t)nis_act_cache_floats(F, B);
+    if (nis_build_dev_flow(desc, &F) != NIS_OK || B < 0 || !nis_flow_plan(F, B, NIS_BN_TRAIN).act_cache) return 0;
+    const size_t tiles = (size_t)((B + 127) / 128);
+    return (int64_t)((size_t)F.n_cells * F.depth * tiles * F.widths[0] * 128);
 }
-
-// The fp16-split kernel (flow_tc_h.cu) runs the width-64 PWLin / PWQuad flows with 32 bins that nis_tc_supported accepts,
-// the gate of the tensor-core backward; nis_h_supported accepts all of them.  On its own it would accept about five times
-// as many shapes (for example every n_flow >= 10 at depth 1), which run on the streamed-weights kernel (flow_wide.cu) today:
-// giving them to the fp16-split kernel needs parity tests and B200 timings against that kernel of their own.
-static bool h_path(const DevFlow& F, int64_t B, int bn_mode) { return nis_tc_supported(F, B, bn_mode) && nis_h_supported(F, B, bn_mode); }
 
 // One cell on the fp16-split kernel, forward or inverse (A.inverse).  Train mode: BN_0 and BN_1 from the column moments
 // unless the previous cell's final pass has taken them (moments_ready), then a layer pass per remaining BN layer.  With
@@ -498,6 +486,55 @@ static int h_cell(const DevFlow& F, FwdArgs& A, const FlowWorkspace& ws, int bn_
     return NIS_OK;
 }
 
+// One train-mode cell on the shape-generic kernel, forward or inverse (A.inverse): a statistics pass per BN layer, then the
+// final pass.  It reads the state rows from state_in (nullptr: the input rows A.in) and writes them to state_out and, with
+// to_out, to A.out.
+static int generic_cell(const DevFlow& F, FwdArgs& A, int c, const float* state_in, float* state_out, bool to_out,
+                        cudaStream_t s) {
+    A.c_begin = c; A.c_end = c + 1;
+    A.from_state = state_in != nullptr; A.state_in = state_in;
+    A.state_out = nullptr; A.to_out = 0;
+    int rc;
+    for (int l = 0; l <= F.depth; ++l) {
+        A.stats_layer = l;
+        rc = launch_fwd_any(F, A, s);
+        if (rc) return rc;
+        timing_mark(s, 2);
+    }
+    A.stats_layer = -1;
+    A.state_out = state_out; A.to_out = to_out;
+    rc = launch_fwd_any(F, A, s);
+    if (rc) return rc;
+    timing_mark(s, 2);
+    return NIS_OK;
+}
+
+// Start of nis_flow_forward and nis_flow_inverse: checks the arguments, carves the workspace, zeroes the last-block ticket,
+// packs the weights (wpack) and fills the fields of A that both calls set alike.  B == 0 returns NIS_OK with nothing launched.
+static int fwd_prologue(const NisFlowDesc* desc, const float* params, const float* bn_running, const void* in, int in_dtype,
+                        int in_cols, void* out, int out_dtype, int bn_mode, void* workspace, size_t workspace_bytes, int64_t B,
+                        cudaStream_t s, DevFlow& F, FlowWorkspace& ws, FwdArgs& A) {
+    int rc = nis_build_dev_flow(desc, &F);
+    if (rc) return rc;
+    if (!params || !workspace || B < 0 || (B > 0 && (!in || !out))) return NIS_EINVAL;
+    if (in_cols != F.d && in_cols != F.d + 1) return NIS_EINVAL;
+    if ((in_dtype != NIS_F32 && in_dtype != NIS_F64) || (out_dtype != NIS_F32 && out_dtype != NIS_F64)) return NIS_EINVAL;
+    if (bn_mode == NIS_BN_EVAL && !bn_running) return NIS_EINVAL;
+    if (workspace_bytes < nis_flow_workspace_bytes(desc, B)) return NIS_EWORKSPACE;
+    if (B == 0) return NIS_OK;
+    nis_flow_carve(F, B, workspace, &ws);
+    cudaMemsetAsync(ws.counter, 0, 256, s);
+    timing_mark(s, -1);                     // open the first interval on this stream (after the counter memset)
+    rc = launch_flow_pack(F, params, bn_running, ws.wpack, bn_mode, s);
+    if (rc) return rc;
+    timing_mark(s, 0);
+    A.in = in; A.in_dtype = in_dtype; A.in_cols = in_cols;
+    A.out = out; A.out_dtype = out_dtype;
+    A.params = params; A.wpack = ws.wpack;
+    A.partials = ws.partials; A.counter = ws.counter; A.B = B;
+    return NIS_OK;
+}
+
 extern "C" int nis_flow_forward(const NisFlowDesc* desc, const float* params, float* bn_running,
                                 const void* xj_in, int32_t in_dtype, int32_t in_cols,
                                 void* xj_out, int32_t out_dtype, int32_t* bins_out,
@@ -512,41 +549,18 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
                                        void* xj_out, int32_t out_dtype, int32_t* bins_out,
                                        float* saved, float* bn_saved, float* act_saved, int32_t bn_mode,
                                        void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
-    DevFlow F;
-    int rc = nis_build_dev_flow(desc, &F);
-    if (rc) return rc;
-    if (!params || !workspace || B < 0 || (B > 0 && (!xj_in || !xj_out))) return NIS_EINVAL;
-    if (in_cols != F.d && in_cols != F.d + 1) return NIS_EINVAL;
-    if ((in_dtype != NIS_F32 && in_dtype != NIS_F64) || (out_dtype != NIS_F32 && out_dtype != NIS_F64)) return NIS_EINVAL;
-    if (bn_mode == NIS_BN_EVAL && !bn_running) return NIS_EINVAL;
-    if (workspace_bytes < nis_flow_workspace_bytes(desc, B)) return NIS_EWORKSPACE;
-    if (B == 0) return NIS_OK;
     cudaStream_t s = (cudaStream_t)stream;
+    DevFlow F;
     FlowWorkspace ws;
-    nis_flow_carve(F, B, workspace, &ws);
-    cudaMemsetAsync(ws.counter, 0, 256, s);
-    {
-        int mx = 0;
-        for (int c = 0; c < F.n_cells; ++c) {
-            int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
-            if (sz > mx) mx = sz;
-        }
-        int bx = (mx + 255) / 256;
-        if (bx > 64) bx = 64;
-        timing_mark(s, -1);                 // open the first interval on this stream (after the counter memset)
-        flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, bn_mode);
-        NIS_CUDA_CHECK_LAUNCH();
-        timing_mark(s, 0);
-    }
     FwdArgs A;
-    A.in = xj_in; A.in_dtype = in_dtype; A.in_cols = in_cols;
-    A.out = xj_out; A.out_dtype = out_dtype;
-    A.saved = saved; A.bins = bins_out;
-    A.params = params; A.wpack = ws.wpack; A.bn_running = bn_running; A.bn_saved = bn_saved;
-    A.partials = ws.partials; A.counter = ws.counter; A.B = B;
-    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 0; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
+    int rc = fwd_prologue(desc, params, bn_running, xj_in, in_dtype, in_cols, xj_out, out_dtype, bn_mode, workspace,
+                          workspace_bytes, B, s, F, ws, A);
+    if (rc || B == 0) return rc;
+    A.saved = saved; A.bins = bins_out; A.bn_running = bn_running; A.bn_saved = bn_saved;
     const long long rows = (long long)B * (F.d + 1);
-    if (h_path(F, B, bn_mode)) {
+    const bool train = bn_mode == NIS_BN_TRAIN;
+    const FlowPlan plan = nis_flow_plan(F, B, bn_mode);
+    if (plan.fwd == FWD_H) {
         rc = nis_h_pack(F, params, ws.tcpack, s);
         if (rc) return rc;
         timing_mark(s, 0);
@@ -559,33 +573,33 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
         }
         return NIS_OK;
     }
-    // every other shape: streamed-weights tcgen05 kernel (flow_wide.cu), else the FP32 register-tiled kernel, else the
-    // shape-generic one
-    const bool wide = nis_wide_supported(F, B, bn_mode);
-    const bool tiled = wide || nis_tiled_supported(F, B);
-    if (wide) { rc = nis_wide_pack(F, params, ws.tcpack, s); if (rc) return rc; }
-    if (bn_mode == NIS_BN_EVAL && !tiled) {
-        A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 1;
-        A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
-        return launch_fwd_any(F, A, s);
-    }
-    if (bn_mode == NIS_BN_TRAIN && !tiled) {
-        // small batch: every pass of every cell inside one cooperative launch (falls through when not co-resident)
-        static const int coop_env = [] { const char* e = getenv("NIS_COOP"); return e && e[0] == '0' ? 0 : 1; }();
-        if (coop_env) {
-            A.scratch_state = ws.state;
-            A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 0;
-            A.c_begin = 0; A.c_end = 1; A.stats_layer = 0;
-            rc = launch_fwd_coop(F, A, s);
-            if (rc == NIS_OK) { timing_mark(s, 2); return NIS_OK; }
+    if (plan.fwd == FWD_GENERIC) {
+        if (!train) {
+            A.to_out = 1; A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
+            return launch_fwd_any(F, A, s);
         }
+        // small batch: every pass of every cell inside one cooperative launch, else one launch sequence per cell
+        A.scratch_state = ws.state;
+        A.c_begin = 0; A.c_end = 1; A.stats_layer = 0;
+        rc = launch_fwd_coop(F, A, s);
+        if (rc == NIS_OK) { timing_mark(s, 2); return NIS_OK; }
+        for (int c = 0; c < F.n_cells; ++c) {
+            const bool last = c == F.n_cells - 1;
+            rc = generic_cell(F, A, c, c > 0 ? (saved ? saved + c * rows : ws.state) : nullptr,
+                              saved ? saved + (c + 1) * rows : (last ? nullptr : ws.state), last, s);
+            if (rc) return rc;
+        }
+        return NIS_OK;
     }
+    // streamed-weights tcgen05 kernel (flow_wide.cu) or FP32 register-tiled kernel (flow_tiled.cu)
+    const bool wide = plan.fwd == FWD_WIDE;
+    if (wide) { rc = nis_wide_pack(F, params, ws.tcpack, s); if (rc) return rc; }
     // activation cache (nis_flow_forward_cached): the wide layer passes write z_1..z_depth of every cell there instead of the
     // two rotating workspace buffers
-    float* acts = (wide && bn_mode == NIS_BN_TRAIN && act_saved && saved && nis_act_cache_floats(F, B)) ? act_saved : nullptr;
+    float* acts = (plan.act_cache && act_saved && saved) ? act_saved : nullptr;
     const size_t act_layer = (size_t)((B + 127) / 128) * (size_t)F.widths[0] * 128;
-    // One launch sequence per cell.  TRAIN: a statistics pass per BN layer, then the full pass.
-    // (EVAL reaches here only on the register-tiled and streamed-weights paths, whose launches are per cell.)
+    // One launch sequence per cell.  TRAIN: the statistics of BN_0 (and BN_1), a layer pass per remaining BN layer, then
+    // the final pass.  EVAL: on the wide kernel a layer pass per hidden layer after the first, then the final pass.
     for (int c = 0; c < F.n_cells; ++c) {
         A.c_begin = c; A.c_end = c + 1;
         A.from_state = c > 0;
@@ -595,8 +609,8 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
         float* const acell = acts ? acts + (size_t)c * F.depth * act_layer : nullptr;
         // BN0 + BN1 from one streaming pass over the pass-through columns (flow_col_moments_kernel), then
         // the layer passes start at layer 2 (recomputing the K=P layer 0 on the way)
-        const bool moments = tiled && bn_mode == NIS_BN_TRAIN && nis_moments_supported(F, c);
-        if (bn_mode == NIS_BN_TRAIN) {
+        const bool moments = train && nis_moments_supported(F, c);
+        if (train) {
             int l0 = 0;
             if (moments) {
                 A.stats_layer = 0;
@@ -607,7 +621,7 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
             }
             for (int l = l0; l <= F.depth; ++l) {
                 A.stats_layer = l;
-                if (tiled && l >= 1) {
+                if (l >= 1) {
                     // layer pass: reads the pre-BN activations of layer l-1, writes those of layer l
                     A.zin = (l >= 2 && !(moments && l == 2)) ? zb[(l - 1) & 1] : nullptr;
                     A.zout = zb[l & 1];
@@ -617,20 +631,18 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
                         A.z1out = (!A.zin && l == 2) ? acell : nullptr;
                     }
                     rc = wide ? nis_launch_wide(F, A, ws.tcpack, s) : nis_launch_tiled(F, A, s);
-                } else if (tiled && l == 0) {
-                    rc = nis_launch_col_stats(F, A, s);
                 } else {
-                    rc = launch_fwd_any(F, A, s);
+                    rc = nis_launch_col_stats(F, A, s);
                 }
                 if (rc) return rc;
                 timing_mark(s, wide && l >= 1 ? 10 + 1 + (A.zin ? 2 : 0) : 2);
             }
         }
         A.stats_layer = -1;
-        A.zin = (tiled && bn_mode == NIS_BN_TRAIN && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
+        A.zin = (train && !(moments && F.depth == 1)) ? zb[F.depth & 1] : nullptr;
         A.zout = nullptr;
         if (acell) { A.zin = acell + (size_t)(F.depth - 1) * act_layer; A.z1out = nullptr; }
-        if (wide && bn_mode == NIS_BN_EVAL) {
+        if (wide && !train) {
             // eval, wide conditioner: one launch per hidden layer (no statistics), then the final pass
             A.no_stats = 1;
             for (int l = 2; l <= F.depth; ++l) {
@@ -645,7 +657,7 @@ extern "C" int nis_flow_forward_cached(const NisFlowDesc* desc, const float* par
         const bool last = c == F.n_cells - 1;
         A.to_out = last;
         A.state_out = saved ? saved + (long long)(c + 1) * rows : (last ? nullptr : ws.state);
-        rc = wide ? nis_launch_wide(F, A, ws.tcpack, s) : tiled ? nis_launch_tiled(F, A, s) : launch_fwd_any(F, A, s);
+        rc = wide ? nis_launch_wide(F, A, ws.tcpack, s) : nis_launch_tiled(F, A, s);
         if (rc) return rc;
         timing_mark(s, wide ? 10 + (A.zin ? 2 : 0) : 2);
     }
@@ -678,40 +690,15 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
                                 const void* yj_in, int32_t in_dtype, int32_t in_cols,
                                 void* xj_out, int32_t out_dtype, int32_t* bins_out, int32_t bn_mode,
                                 void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
-    DevFlow F;
-    int rc = nis_build_dev_flow(desc, &F);
-    if (rc) return rc;
-    if (!params || !workspace || B < 0 || (B > 0 && (!yj_in || !xj_out))) return NIS_EINVAL;
-    if (in_cols != F.d && in_cols != F.d + 1) return NIS_EINVAL;
-    if ((in_dtype != NIS_F32 && in_dtype != NIS_F64) || (out_dtype != NIS_F32 && out_dtype != NIS_F64)) return NIS_EINVAL;
-    if (bn_mode == NIS_BN_EVAL && !bn_running) return NIS_EINVAL;
-    if (workspace_bytes < nis_flow_workspace_bytes(desc, B)) return NIS_EWORKSPACE;
-    if (B == 0) return NIS_OK;
     cudaStream_t s = (cudaStream_t)stream;
+    DevFlow F;
     FlowWorkspace ws;
-    nis_flow_carve(F, B, workspace, &ws);
-    cudaMemsetAsync(ws.counter, 0, 256, s);
-    {
-        int mx = 0;
-        for (int c = 0; c < F.n_cells; ++c) {
-            int sz = (c + 1 < F.n_cells ? F.cells[c + 1].pk_off : F.pack_total) - F.cells[c].pk_off;
-            if (sz > mx) mx = sz;
-        }
-        int bx = (mx + 255) / 256;
-        if (bx > 64) bx = 64;
-        timing_mark(s, -1);
-        flow_pack_kernel<<<dim3(bx, F.n_cells), 256, 0, s>>>(F, params, bn_running, ws.wpack, bn_mode);
-        NIS_CUDA_CHECK_LAUNCH();
-        timing_mark(s, 0);
-    }
     FwdArgs A;
-    A.in = yj_in; A.in_dtype = in_dtype; A.in_cols = in_cols;
-    A.out = xj_out; A.out_dtype = out_dtype;
-    A.saved = nullptr; A.bins = bins_out;
-    A.params = params; A.wpack = ws.wpack; A.bn_running = nullptr; A.bn_saved = nullptr;
-    A.partials = ws.partials; A.counter = ws.counter; A.B = B;
-    A.zin = nullptr; A.zout = nullptr; A.no_stats = 0; A.z1out = nullptr; A.scratch_state = nullptr; A.inverse = 1; A.zin_layer = 0; A.next_moments = 0; A.next_cell = 0;
-    if (h_path(F, B, bn_mode)) {
+    int rc = fwd_prologue(desc, params, bn_running, yj_in, in_dtype, in_cols, xj_out, out_dtype, bn_mode, workspace,
+                          workspace_bytes, B, s, F, ws, A);
+    if (rc || B == 0) return rc;
+    A.bins = bins_out; A.inverse = 1;
+    if (nis_flow_plan(F, B, bn_mode).fwd == FWD_H) {
         // the forward's launch sequence with the cells in reverse order, from float32 state rows in the physical column
         // order.  The statistics and layer passes are the forward's (they read only the pass-through columns); the fused
         // cell and the final pass run the inverse splines; the fused column moments of a final pass are those of cell c - 1.
@@ -730,29 +717,14 @@ extern "C" int nis_flow_inverse(const NisFlowDesc* desc, const float* params, co
         return NIS_OK;
     }
     if (bn_mode == NIS_BN_EVAL) {
-        A.state_in = nullptr; A.state_out = nullptr; A.from_state = 0; A.to_out = 1;
-        A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
+        A.to_out = 1; A.c_begin = 0; A.c_end = F.n_cells; A.stats_layer = -1;
         rc = launch_fwd_any(F, A, s);
         if (rc == NIS_OK) timing_mark(s, 2);
         return rc;
     }
     for (int c = F.n_cells - 1; c >= 0; --c) {
-        A.c_begin = c; A.c_end = c + 1;
-        A.from_state = c < F.n_cells - 1;
-        A.state_in = A.from_state ? ws.state : nullptr;
-        A.state_out = nullptr; A.to_out = 0;
-        for (int l = 0; l <= F.depth; ++l) {
-            A.stats_layer = l;
-            rc = launch_fwd_any(F, A, s);
-            if (rc) return rc;
-            timing_mark(s, 2);
-        }
-        A.stats_layer = -1;
-        A.to_out = c == 0;
-        A.state_out = c == 0 ? nullptr : ws.state;
-        rc = launch_fwd_any(F, A, s);
+        rc = generic_cell(F, A, c, c < F.n_cells - 1 ? ws.state : nullptr, c == 0 ? nullptr : ws.state, c == 0, s);
         if (rc) return rc;
-        timing_mark(s, 2);
     }
     return NIS_OK;
 }

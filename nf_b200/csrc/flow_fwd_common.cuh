@@ -1,31 +1,35 @@
 // Pieces shared by the forward kernels (flow_fwd.cu: shape-generic; flow_tiled.cu: register-tiled).
 #pragma once
+#include <type_traits>
 #include "common.cuh"
 
+// (default member initialisers: a caller sets only what its launches use; the struct stays trivially copyable, it is a
+// __grid_constant__ kernel argument)
 struct FwdArgs {
-    const void* in; int in_dtype; int in_cols;   // external input rows (first cell, !from_state)
-    const float* state_in;                       // fp32 [B][d+1] (from_state)
-    float* state_out;                            // fp32 [B][d+1] or null
-    void* out; int out_dtype;                    // external output (to_out)
-    int from_state, to_out;
-    float* saved;                                // [n_cells+1][B][d+1] or null
-    int32_t* bins;
-    const float* params; float* wpack; float* bn_running; float* bn_saved;
-    double* partials; unsigned* counter;
-    long long B; int c_begin, c_end, stats_layer;
-    const float* zin;                            // tiled train path: pre-BN activations of the layer below,
-    float* zout;                                 // tile-blocked [tile][64][M] (written by a statistics pass)
-    int no_stats;                                // layer pass that only stores its activations (eval-mode split cell)
-    float* z1out;                          // wide kernel, pass from the state: also store z_1 (backward recompute) or null
-    float* scratch_state;                  // cooperative small-batch kernel: fp32 [B][d+1] state between cells when `saved` is null
-    int zin_layer;                         // fp16-split kernel: which layer's pre-activations `zin` holds (0: the default,
+    const void* in = nullptr; int in_dtype = NIS_F32; int in_cols = 0;   // external input rows (first cell, !from_state)
+    const float* state_in = nullptr;             // fp32 [B][d+1] (from_state)
+    float* state_out = nullptr;                  // fp32 [B][d+1] or null
+    void* out = nullptr; int out_dtype = NIS_F32;    // external output (to_out)
+    int from_state = 0, to_out = 0;
+    float* saved = nullptr;                      // [n_cells+1][B][d+1] or null
+    int32_t* bins = nullptr;
+    const float* params = nullptr; float* wpack = nullptr; float* bn_running = nullptr; float* bn_saved = nullptr;
+    double* partials = nullptr; unsigned* counter = nullptr;
+    long long B = 0; int c_begin = 0, c_end = 0, stats_layer = -1;
+    const float* zin = nullptr;                  // tiled train path: pre-BN activations of the layer below,
+    float* zout = nullptr;                       // tile-blocked [tile][64][M] (written by a statistics pass)
+    int no_stats = 0;                            // layer pass that only stores its activations (eval-mode split cell)
+    float* z1out = nullptr;                // wide kernel, pass from the state: also store z_1 (backward recompute) or null
+    float* scratch_state = nullptr;        // cooperative small-batch kernel: fp32 [B][d+1] state between cells when `saved` is null
+    int zin_layer = 0;                     // fp16-split kernel: which layer's pre-activations `zin` holds (0: the default,
                                            // stats_layer - 1 for a layer pass, depth for the final pass)
-    int next_moments;                      // fp16-split final pass: also accumulate the column moments of cell next_cell (its
+    int next_moments = 0;                  // fp16-split final pass: also accumulate the column moments of cell next_cell (its
                                            // BN_0 / BN_1 statistics) from the state this pass writes - no pass of their own
-    int next_cell;                         // the cell that runs after c_begin: c_begin + 1, or c_begin - 1 in the inverse
-    int inverse;                           // nis_flow_inverse: cells backwards, inverse splines, J divided (shape-generic
+    int next_cell = 0;                     // the cell that runs after c_begin: c_begin + 1, or c_begin - 1 in the inverse
+    int inverse = 0;                       // nis_flow_inverse: cells backwards, inverse splines, J divided (shape-generic
                                            // kernel; fp16-split fused cell and final pass)
 };
+static_assert(std::is_trivially_copyable<FwdArgs>::value, "FwdArgs is a kernel argument");
 
 
 __device__ __forceinline__ float load_io(const void* p, int dtype, long long idx) {

@@ -652,12 +652,6 @@ size_t nis_h_pack_floats(const DevFlow& F) {
     return (size_t)F.n_cells * (h_cell_bytes(F) / 4);
 }
 
-// smallest batch the tensor-core kernels take (below it the shape-generic kernel runs); NIS_TC_MIN_B overrides (test knob)
-int64_t nis_tc_min_batch(int64_t dflt) {
-    const char* e = getenv("NIS_TC_MIN_B");
-    return e ? atoll(e) : dflt;
-}
-
 static int h_groups(const DevFlow& F) {
     // the largest group count whose three launch shapes fit the shared memory of an SM
     const size_t lim = 226 * 1024;
@@ -673,20 +667,6 @@ static int h_groups(const DevFlow& F) {
         if (ok) return ng;
     }
     return 0;
-}
-
-// Width-64 cells with 32 bins: PWLin (BASELINE configs[1]) and PWQuad (configs[3])
-bool nis_h_supported(const DevFlow& F, int64_t B, int bn_mode) {
-    (void)bn_mode;
-    const char* tcoff = getenv("NIS_TC");
-    if (tcoff && tcoff[0] == '0') return false;
-    if (F.nb != 32 || F.depth < 1 || F.maxW != TCH) return false;
-    if (F.kind == NIS_KIND_PWLIN ? F.K != 32 : F.K != 65) return false;
-    if (B < nis_tc_min_batch(256)) return false;
-    for (int l = 0; l < F.depth; ++l) if (F.widths[l] != TCH) return false;
-    for (int c = 0; c < F.n_cells; ++c)
-        if (F.cells[c].P > 16 || (F.kind == NIS_KIND_PWLIN && F.cells[c].T * 32 > 128)) return false;
-    return h_groups(F) >= 2;
 }
 
 int nis_h_pack(const DevFlow& F, const float* params, float* tcpack, cudaStream_t s) {
@@ -726,13 +706,7 @@ static int h_launch(const DevFlow& F, const FwdArgs& A, const char* hpack, size_
 }
 
 int nis_launch_h(const DevFlow& F, const FwdArgs& A, const float* tcpack, cudaStream_t s) {
-    static int sms = 0;
-    if (sms <= 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (sms <= 0) sms = 148;
-    }
+    const int sms = nis_sm_count();
     const bool stats = A.stats_layer >= 1;
     const int lz = A.zin ? (A.zin_layer > 0 ? A.zin_layer : (stats ? A.stats_layer - 1 : F.depth)) : 1;
     const int l_end = stats ? A.stats_layer - 1 : F.depth;

@@ -14,6 +14,7 @@
 #include "common.cuh"
 #include "spline.cuh"
 #include "flow_fwd_common.cuh"
+#include "flow_host.cuh"
 
 #define TH 64            // hidden width handled by this path
 #define TCH 64           // logits per output-layer chunk
@@ -470,10 +471,8 @@ int nis_launch_col_stats(const DevFlow& F, const FwdArgs& A, cudaStream_t s) {
 
 size_t nis_tiled_zbuf_floats(int64_t B) { return (size_t)((B + 255) / 256) * 256 * TH; }
 
-bool nis_tiled_supported(const DevFlow& F, int64_t B) {
-    const char* off = getenv("NIS_DISABLE_TILED");        // test knob: force the shape-generic kernel
-    if (off && off[0] == '1') return false;
-    if (F.kind != NIS_KIND_PWLIN || F.depth < 1 || B < 2048) return false;
+bool nis_tiled_supported(const DevFlow& F) {
+    if (F.kind != NIS_KIND_PWLIN || F.depth < 1) return false;
     for (int l = 0; l < F.depth; ++l) if (F.widths[l] != TH) return false;
     if (F.K != 8 && F.K != 16 && F.K != 32 && F.K != 64) return false;
     if (F.maxW != TH) return false;
@@ -501,10 +500,7 @@ static int launch_tiled_m(const DevFlow& F, const FwdArgs& A, int sms, cudaStrea
 }
 
 int nis_launch_tiled(const DevFlow& F, const FwdArgs& A, cudaStream_t s) {
-    int sms = 0, dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
+    const int sms = nis_sm_count();
     // train-mode layer passes exchange tile-blocked activations: every launch of a forward must use the
     // same M; they run at M=128 with two CTAs per SM.  The fused eval cell runs at M=256.
     const bool layer_pass = A.zin || A.zout;

@@ -26,6 +26,7 @@
 #include "spline.cuh"
 #include "tc_common.cuh"
 #include "flow_fwd_common.cuh"
+#include "flow_host.cuh"
 
 #include "wide_common.cuh"
 
@@ -378,15 +379,12 @@ __global__ void __launch_bounds__(WD_THREADS, 1) flow_wide_tc_kernel(const __gri
 }
 
 // ---------------------------------------------------------------------------------------------------
-bool nis_moments_supported(const DevFlow& F, int c);
-int64_t nis_tc_min_batch(int64_t dflt);
+// first hidden width of the streamed-weights kernels: 64, 128, 192 or 256
+static bool wide_width(const DevFlow& F) { return F.depth >= 1 && F.widths[0] >= 64 && F.widths[0] <= 256 && !(F.widths[0] & 63); }
 
-bool nis_wide_supported(const DevFlow& F, int64_t B, int bn_mode) {
-    const char* off = getenv("NIS_TC");                   // NIS_TC=0 forces the FP32-pipe kernels (test knob)
-    if (off && off[0] == '0') return false;
-    if (F.depth < 1 || B < nis_tc_min_batch(256) || F.kind == NIS_KIND_AFFINE) return false;
+bool nis_wide_supported(const DevFlow& F, int bn_mode) {
+    if (F.kind == NIS_KIND_AFFINE || !wide_width(F)) return false;  // (width 64 with 32 bins is taken by flow_tc_h.cu first where it applies)
     const int W = F.widths[0];
-    if (W < 64 || W > 256 || (W & 63)) return false;          // (width 64 with 32 bins is taken by flow_tc_h.cu first where it applies)
     for (int l = 0; l < F.depth; ++l) if (F.widths[l] != W) return false;
     if (F.maxW != W) return false;
     if (wd_kp16(F) > WD_NMAX) return false;
@@ -399,10 +397,7 @@ bool nis_wide_supported(const DevFlow& F, int64_t B, int bn_mode) {
     return true;
 }
 
-size_t nis_wide_pack_floats(const DevFlow& F) {
-    if (F.depth < 1 || F.widths[0] < 64 || (F.widths[0] & 63) || F.widths[0] > 256) return 0;
-    return (size_t)F.n_cells * wd_cell_floats(F);
-}
+size_t nis_wide_pack_floats(const DevFlow& F) { return wide_width(F) ? (size_t)F.n_cells * wd_cell_floats(F) : 0; }
 
 int nis_wide_pack(const DevFlow& F, const float* params, float* widepack, cudaStream_t s) {
     flow_wide_pack_kernel<<<dim3(128, F.n_cells), 256, 0, s>>>(F, params, widepack);
@@ -411,10 +406,7 @@ int nis_wide_pack(const DevFlow& F, const float* params, float* widepack, cudaSt
 }
 
 int nis_launch_wide(const DevFlow& F, const FwdArgs& A, const float* widepack, cudaStream_t s) {
-    int sms = 0, dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
+    const int sms = nis_sm_count();
     const bool final_pass = A.stats_layer < 1;
     const WdSmem L = wd_layout(F, F.cells[A.c_begin].P, final_pass, A.zin == nullptr);
     const size_t smem = (size_t)L.total + 1024;

@@ -56,10 +56,7 @@ __global__ void __launch_bounds__(128, 1) mma_rate_kernel(int N, int iters) {
 
 extern "C" int64_t nis_probe_tensor(int32_t kind, int32_t n, int32_t iters, void* stream) {
     if ((kind != 0 && kind != 1) || (n != 64 && n != 128 && n != 256) || iters <= 0 || iters > (1 << 16)) return NIS_EINVAL;
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
+    const int sms = nis_sm_count();
     const int smem = 256 * 128 + 1024;
     cudaStream_t s = (cudaStream_t)stream;
     if (kind == 0) {

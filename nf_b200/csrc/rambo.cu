@@ -95,12 +95,7 @@ static int rambo_launch(const RamboConst& C, const void* r, double* momenta, dou
     NIS_ENSURE_SMEM((rambo_kernel<RT>), (int)smem);
     long long ntiles = (B + RAMBO_NT - 1) / RAMBO_NT;
     // one resident wave: every CTA strides over the same number of tiles (+-1), no partial last wave
-    static int sms = 0;
-    if (sms <= 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
-    }
+    const int sms = nis_sm_count();
     int per_sm = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rambo_kernel<RT>, RAMBO_NT, smem) != cudaSuccess || per_sm < 1)
         per_sm = 4;
