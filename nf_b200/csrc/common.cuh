@@ -39,6 +39,14 @@ static inline int nis_sm_count() {
 static inline __host__ __device__ int pad8(int x) { return (x + 7) & ~7; }
 static inline __host__ __device__ int pad4(int x) { return (x + 3) & ~3; }
 
+// element idx of an external f32 / f64 array (NIS_F32 / NIS_F64): the flow's input and output rows, grad_out and grad_in
+__device__ __forceinline__ float load_io(const void* p, int dtype, long long idx) {
+    return dtype == NIS_F64 ? (float)reinterpret_cast<const double*>(p)[idx] : reinterpret_cast<const float*>(p)[idx];
+}
+__device__ __forceinline__ void store_io(void* p, int dtype, long long idx, float v) {
+    if (dtype == NIS_F64) reinterpret_cast<double*>(p)[idx] = (double)v; else reinterpret_cast<float*>(p)[idx] = v;
+}
+
 // Device-side view of one coupling cell: column tables + offsets into the three float arenas
 //   params      (torch layout, read-only)
 //   bn_running  (running mean/var)

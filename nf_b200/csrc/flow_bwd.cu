@@ -60,8 +60,7 @@ __host__ __device__ static inline int wb_layer_off(const DevFlow& F, int c, int 
     return n;
 }
 
-__global__ void flow_bwd_pack_kernel(DevFlow F, const float* __restrict__ params, float* __restrict__ wb,
-                                     const float* __restrict__ bn_saved, float* __restrict__ wpack, int train) {
+__global__ void flow_bwd_pack_kernel(DevFlow F, const float* __restrict__ params, float* __restrict__ wb) {
     const int c = blockIdx.y;
     const DevCell& q = F.cells[c];
     const float* p = params + q.param_off;
@@ -80,19 +79,6 @@ __global__ void flow_bwd_pack_kernel(DevFlow F, const float* __restrict__ params
             dst[i] = k < in ? w[(long long)src * in + k] : 0.f;
         }
         if (l < F.depth) in = F.widths[l];
-    }
-    if (train) {   // BN scale/shift of THIS forward's batch statistics (wpack may hold a later batch's)
-        for (int l = 0; l <= F.depth; ++l) {
-            const int W = F.W(c, l), Wp = F.Wp(c, l);
-            const long long g = F.p_bn_gamma(c, l);
-            const float* sv = bn_saved + q.sv_off + l * 2 * F.maxW;
-            float* aff = wpack + q.pk_off + q.aff_off[l];
-            for (int j = tid; j < Wp; j += nth) {
-                float sc = 0.f, sh = 0.f;
-                if (j < W) { sc = p[g + j] * sv[F.maxW + j]; sh = p[g + W + j] - sv[j] * sc; }
-                aff[j] = sc; aff[Wp + j] = sh;
-            }
-        }
     }
 }
 
@@ -162,10 +148,6 @@ __device__ __forceinline__ void rowsum_accum(const float* buf, int J, float* gv)
     }
 }
 
-__device__ __forceinline__ float load_g(const void* p, int dtype, long long idx) {
-    return dtype == NIS_F64 ? (float)reinterpret_cast<const double*>(p)[idx] : reinterpret_cast<const float*>(p)[idx];
-}
-
 template <int NT>
 __device__ __forceinline__ void bwd_generic_body(const DevFlow& F, const BwdArgs& A, float* sm) {
     const int tid = threadIdx.x;
@@ -219,8 +201,8 @@ __device__ __forceinline__ void bwd_generic_body(const DevFlow& F, const BwdArgs
             for (int i = 0; i <= d; ++i) st[i * NT] = sv[i];
             Jout = A.saved[((long long)(c + 1) * A.B + pt) * rowlen + d];
             if (A.step_begin == OUT && A.first) {
-                for (int i = 0; i < d; ++i) g[F.out_perm[i] * NT] = load_g(A.grad_out, A.grad_dtype, pt * rowlen + i);
-                g[d * NT] = load_g(A.grad_out, A.grad_dtype, pt * rowlen + d);
+                for (int i = 0; i < d; ++i) g[F.out_perm[i] * NT] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + i);
+                g[d * NT] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + d);
             } else {
                 for (int i = 0; i <= d; ++i) g[i * NT] = A.gstate[pt * rowlen + i];
             }
@@ -398,12 +380,8 @@ __device__ __forceinline__ void bwd_generic_body(const DevFlow& F, const BwdArgs
         }
         // ---- store the gradient state ------------------------------------------------------------
         if (valid && (A.step_begin == OUT || A.step_end == 0)) {
-            if (A.grad_in && A.step_end == 0) {
-                for (int i = 0; i <= d; ++i) {
-                    if (A.grad_dtype == NIS_F64) reinterpret_cast<double*>(A.grad_in)[pt * rowlen + i] = (double)g[i * NT];
-                    else reinterpret_cast<float*>(A.grad_in)[pt * rowlen + i] = g[i * NT];
-                }
-            }
+            if (A.grad_in && A.step_end == 0)
+                for (int i = 0; i <= d; ++i) store_io(A.grad_in, A.grad_dtype, pt * rowlen + i, g[i * NT]);
             for (int i = 0; i <= d; ++i) A.gstate[pt * rowlen + i] = g[i * NT];
         }
     }
@@ -566,47 +544,18 @@ static int launch_bwd_any(const DevFlow& F, const BwdArgs& A, int NT, int grid, 
     return NIS_EUNSUPPORTED;
 }
 
-extern "C" int nis_flow_backward(const NisFlowDesc* desc, const float* params, const float* bn_running,
-                                 const float* saved, const float* bn_saved, const void* grad_out,
-                                 int32_t grad_dtype, float* grad_params, void* grad_in, int32_t bn_mode,
-                                 void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
-    return nis_flow_backward_cached(desc, params, bn_running, saved, bn_saved, nullptr, grad_out, grad_dtype, grad_params,
-                                    grad_in, bn_mode, workspace, workspace_bytes, B, stream);
-}
-
-extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* params, const float* bn_running,
-                                        const float* saved, const float* bn_saved, const float* act_saved,
-                                        const void* grad_out, int32_t grad_dtype, float* grad_params, void* grad_in,
-                                        int32_t bn_mode, void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
-    DevFlow F;
-    int rc = nis_build_dev_flow(desc, &F);
-    if (rc) return rc;
-    if (!params || !saved || !grad_out || !grad_params || !workspace || B < 0) return NIS_EINVAL;
-    if (grad_dtype != NIS_F32 && grad_dtype != NIS_F64) return NIS_EINVAL;
+// Shape-generic backward, train or eval mode: one launch per step of each cell (train), one per cell (eval), or the whole
+// backward in one cooperative launch.
+static int nis_flow_backward_generic(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* saved,
+                                     int bn_mode, const void* grad_out, int grad_dtype, float* grad_params, void* grad_in,
+                                     int64_t B, cudaStream_t s) {
     const int train = bn_mode == NIS_BN_TRAIN;
-    if (train && !bn_saved) return NIS_EINVAL;
-    if (!train && !bn_running) return NIS_EINVAL;
-    if (workspace_bytes < nis_flow_workspace_bytes(desc, B)) return NIS_EWORKSPACE;
-    if (B == 0) return NIS_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    FlowWorkspace ws;
-    nis_flow_carve(F, B, workspace, &ws);
-    const FlowPlan plan = nis_flow_plan(F, B, bn_mode);
-    if (plan.bwd == BWD_TC)
-        return nis_flow_backward_tc(F, ws, params, bn_running, saved, bn_saved, grad_out, grad_dtype, grad_params, grad_in, B, s);
-    if (plan.bwd == BWD_WIDE)
-        return nis_flow_backward_wide(F, ws, params, bn_running, saved, bn_saved, plan.act_cache ? act_saved : nullptr,
-                                      grad_out, grad_dtype, grad_params, grad_in, B, s);
     bool rotate = false;
     const int NT = bwd_pick_nt(F, train != 0, &rotate);
-    if (!NT) return NIS_EUNSUPPORTED;
     BwdScratch sc;
     bwd_carve(F, B, ws.bwd, &sc);
     const int grid = bwd_grid(F, B, NT);
-    cudaMemsetAsync(ws.counter, 0, 256, s);
-    rc = launch_flow_pack(F, params, bn_running, ws.wpack, bn_mode, s);
-    if (rc) return rc;
-    flow_bwd_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, sc.wb, bn_saved, ws.wpack, train);
+    flow_bwd_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, sc.wb);
     NIS_CUDA_CHECK_LAUNCH();
     BwdArgs A;
     A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype;
@@ -614,6 +563,7 @@ extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* pa
     A.bnb = sc.bnb; A.gpart = sc.gpart; A.grad_params = grad_params;
     A.partials = ws.partials; A.counter = ws.counter; A.B = B; A.train = train; A.rotate = rotate;
     const int OUT = F.depth + 1;
+    int rc;
     if (train && NT == 128 && !rotate) {
         // small batch: the whole backward in one cooperative launch when every tile has its own resident CTA
         const long long ntiles = (B + NT - 1) / NT;
@@ -659,4 +609,45 @@ extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* pa
         NIS_CUDA_CHECK_LAUNCH();
     }
     return NIS_OK;
+}
+
+extern "C" int nis_flow_backward(const NisFlowDesc* desc, const float* params, const float* bn_running,
+                                 const float* saved, const float* bn_saved, const void* grad_out,
+                                 int32_t grad_dtype, float* grad_params, void* grad_in, int32_t bn_mode,
+                                 void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
+    return nis_flow_backward_cached(desc, params, bn_running, saved, bn_saved, nullptr, grad_out, grad_dtype, grad_params,
+                                    grad_in, bn_mode, workspace, workspace_bytes, B, stream);
+}
+
+// Checks the arguments and everything that can refuse the call before any launch, then zeroes the last-block ticket and packs
+// the weights and this batch's BN scale/shift (wpack) for whichever backward nis_flow_plan picks.
+extern "C" int nis_flow_backward_cached(const NisFlowDesc* desc, const float* params, const float* bn_running,
+                                        const float* saved, const float* bn_saved, const float* act_saved,
+                                        const void* grad_out, int32_t grad_dtype, float* grad_params, void* grad_in,
+                                        int32_t bn_mode, void* workspace, size_t workspace_bytes, int64_t B, void* stream) {
+    DevFlow F;
+    int rc = nis_build_dev_flow(desc, &F);
+    if (rc) return rc;
+    if (!params || !saved || !grad_out || !grad_params || !workspace || B < 0) return NIS_EINVAL;
+    if (grad_dtype != NIS_F32 && grad_dtype != NIS_F64) return NIS_EINVAL;
+    const int train = bn_mode == NIS_BN_TRAIN;
+    if (train && !bn_saved) return NIS_EINVAL;
+    if (!train && !bn_running) return NIS_EINVAL;
+    if (workspace_bytes < nis_flow_workspace_bytes(desc, B)) return NIS_EWORKSPACE;
+    if (B == 0) return NIS_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    FlowWorkspace ws;
+    nis_flow_carve(F, B, workspace, &ws);
+    const FlowPlan plan = nis_flow_plan(F, B, bn_mode);
+    bool rotate;
+    if (plan.bwd == BWD_GENERIC && !bwd_pick_nt(F, train != 0, &rotate)) return NIS_EUNSUPPORTED;
+    cudaMemsetAsync(ws.counter, 0, 256, s);
+    rc = launch_flow_pack(F, params, bn_running, bn_saved, ws.wpack, bn_mode, s);
+    if (rc) return rc;
+    if (plan.bwd == BWD_TC)
+        return nis_flow_backward_tc(F, ws, params, saved, bn_saved, grad_out, grad_dtype, grad_params, grad_in, B, s);
+    if (plan.bwd == BWD_WIDE)
+        return nis_flow_backward_wide(F, ws, params, saved, bn_saved, plan.act_cache ? act_saved : nullptr, grad_out,
+                                      grad_dtype, grad_params, grad_in, B, s);
+    return nis_flow_backward_generic(F, ws, params, saved, bn_mode, grad_out, grad_dtype, grad_params, grad_in, B, s);
 }

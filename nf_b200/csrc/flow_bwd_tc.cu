@@ -17,7 +17,8 @@
 //            then ReLU mask, store dL/dh_lam, per-feature sums of dL/dh and dL/dh * xhat (recursive-halving
 //            warp shuffles, float64 across tiles, last CTA finalises = dL/dbeta, dL/dgamma and the means the
 //            next launch needs)
-//   tail   : BatchNorm backward of the input normalisation -> dL/dx of the pass-through columns
+//   tail   : BatchNorm backward of the input normalisation -> dL/dx of the pass-through columns (flow_bwd_tail_kernel,
+//            which the wide backward of flow_bwd_wide.cu launches with its own tile stride)
 //
 // 3xTF32 everywhere (hi rounded to nearest, exact residual).  For the wgrad the hi and lo parts of dz are STACKED
 // along M ([dz_hi ; dz_lo], 128 rows) so that two M=128 MMAs (against h_hi and h_lo) give all four partial
@@ -39,7 +40,6 @@
 struct BtArgs {
     const float* saved;                    // [C+1][B][d+1]
     const void* grad_out; int grad_dtype;
-    void* grad_in;
     float* gstate;                         // [B][d+1]
     const float* params; const float* wpack; const float* bn_saved;
     const float* tcpack;                   // forward operands (flow_tc_pack_kernel)
@@ -53,7 +53,6 @@ struct BtArgs {
     double* partials; unsigned* counter;
     long long B, ntiles;
     int c, lam, first, grid;
-    int flush_every;                       // iterations between flushes of the wgrad accumulators (0: only at the end)
 };
 
 // Operands of the head's conditioner recompute: hidden layers 1..depth-1 and the output blocks, each as TF32 hi / lo
@@ -99,10 +98,9 @@ __host__ __device__ static inline int bd_layer_off(const DevFlow& F, int lam) { 
 }
 __host__ __device__ static inline int bd_cell_floats(const DevFlow& F) { return bd_layer_off(F, F.depth) + 2 * 2 * TCH * TCH; }
 
-// dgrad operands + this batch's BN scale/shift.  B operand of "dL/dh = dz W": rows n = input feature i,
-// K = output feature o, i.e. W^T, K-major swizzled; the output layer has K = 128 as two blocks of 64.
-__global__ void flow_bwd_tc_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_saved,
-                                        float* __restrict__ wpack, float* __restrict__ bdpack) {
+// dgrad operands.  B operand of "dL/dh = dz W": rows n = input feature i, K = output feature o, i.e. W^T, K-major swizzled;
+// the output layer has K = 128 as two blocks of 64.
+__global__ void flow_bwd_tc_pack_kernel(DevFlow F, const float* __restrict__ params, float* __restrict__ bdpack) {
     const int c = blockIdx.y;
     const DevCell& q = F.cells[c];
     const float* p = params + q.param_off;
@@ -126,21 +124,6 @@ __global__ void flow_bwd_tc_pack_kernel(DevFlow F, const float* __restrict__ par
             }
         }
     }
-    for (int l = 0; l <= F.depth; ++l) {
-        const int W = F.W(c, l), Wp = F.Wp(c, l);
-        const long long g = F.p_bn_gamma(c, l);
-        const float* sv = bn_saved + q.sv_off + l * 2 * F.maxW;
-        float* aff = wpack + q.pk_off + q.aff_off[l];
-        for (int j = tid; j < Wp; j += nth) {
-            float sc = 0.f, sh = 0.f;
-            if (j < W) { sc = p[g + j] * sv[F.maxW + j]; sh = p[g + W + j] - sv[j] * sc; }
-            aff[j] = sc; aff[Wp + j] = sh;
-        }
-    }
-}
-
-__device__ __forceinline__ float bt_load_g(const void* p, int dtype, long long idx) {
-    return dtype == NIS_F64 ? (float)reinterpret_cast<const double*>(p)[idx] : reinterpret_cast<const float*>(p)[idx];
 }
 
 // ===================================================================================================
@@ -238,8 +221,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) flow_bwd_tc_head_kernel(const _
                 for (int i = 0; i <= d; ++i) st[i * TCM] = sv[i];
                 Jout = A.saved[((long long)(c + 1) * A.B + pt) * rowlen + d];
                 if (A.first) {
-                    for (int i = 0; i < d; ++i) gr[F.out_perm[i] * TCM] = bt_load_g(A.grad_out, A.grad_dtype, pt * rowlen + i);
-                    gr[d * TCM] = bt_load_g(A.grad_out, A.grad_dtype, pt * rowlen + d);
+                    for (int i = 0; i < d; ++i) gr[F.out_perm[i] * TCM] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + i);
+                    gr[d * TCM] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + d);
                 } else {
                     for (int i = 0; i <= d; ++i) gr[i * TCM] = A.gstate[pt * rowlen + i];
                 }
@@ -483,7 +466,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) flow_bwd_tc_layer_kernel(const 
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_s;
     const long long ntiles = A.ntiles, rowlen = d + 1;
-    const int fevery = A.flush_every * 2;                  // in tiles
+    constexpr int fevery = 2 * BT_FLUSH;                   // in tiles
     int nflush = 0;
     double acc1 = 0.0, acc2 = 0.0, accb[NH];
 #pragma unroll
@@ -532,7 +515,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) flow_bwd_tc_layer_kernel(const 
                     if (h < NH - 1) tc_commit(&hdone); else tc_commit(&done[b]);
                 }
                 fresh = false;
-                if (fevery > 0 && ((it + 1) % fevery) == 0 && tile + gridDim.x < ntiles) {
+                if (((it + 1) % fevery) == 0 && tile + gridDim.x < ntiles) {
                     tc_commit(&acc_ready);
                     mbar_wait(&acc_free, pf);
                     pf ^= 1;
@@ -698,7 +681,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) flow_bwd_tc_layer_kernel(const 
                     acc1 += (double)bt_warp_feature_sums32(dv, lane);
                     acc2 += (double)bt_warp_feature_sums32(pr, lane);
                 }
-                if (sub == 0 && fevery > 0 && ((it + 1) % fevery) == 0 && have_n) {
+                if (sub == 0 && ((it + 1) % fevery) == 0 && have_n) {
                     mbar_wait(&acc_ready, pfr);
                     pfr ^= 1;
                     tc_fence_after();
@@ -791,9 +774,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) flow_bwd_tc_layer_kernel(const 
 }
 
 // ===================================================================================================
-// tail: BatchNorm backward of the input normalisation, dL/dx of the pass-through columns
+// tail: BatchNorm backward of the input normalisation, dL/dx of the pass-through columns (both tensor-core backwards)
 // ===================================================================================================
-__global__ void __launch_bounds__(256) flow_bwd_tc_tail_kernel(const __grid_constant__ DevFlow F, const BtArgs A) {
+__global__ void __launch_bounds__(256) flow_bwd_tail_kernel(const __grid_constant__ DevFlow F, const BwdTailArgs A) {
     const int c = A.c;
     const DevCell& q = F.cells[c];
     const int d = F.d, maxW = F.maxW;
@@ -803,23 +786,25 @@ __global__ void __launch_bounds__(256) flow_bwd_tc_tail_kernel(const __grid_cons
     for (long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x; pt < A.B; pt += (long long)gridDim.x * blockDim.x) {
         const float* xs = A.saved + ((long long)c * A.B + pt) * rowlen;
         float* gs = A.gstate + pt * rowlen;
-        const float* da = A.dh_in + (size_t)(pt >> 7) * BT_TILE + (pt & 127);
+        const float* da = A.dh_in + (size_t)(pt >> 7) * A.tile_floats + (pt & 127);
         float g[NIS_MAX_DIM + 1];
         for (int i = 0; i <= d; ++i) g[i] = gs[i];
         for (int k = 0; k < q.P; ++k) {
             const int col = q.feed[k];
             const float xh = (xs[col] - sv[k]) * sv[maxW + k];
-            const float dz = pk[q.aff_off[0] + k] * (da[(size_t)k * TCM] - A.bnb[k] - xh * A.bnb[maxW + k]);
-            g[col] += dz;
+            g[col] += pk[q.aff_off[0] + k] * (da[(size_t)k * TCM] - A.bnb[k] - xh * A.bnb[maxW + k]);
         }
         for (int i = 0; i <= d; ++i) gs[i] = g[i];
-        if (A.grad_in) {
-            for (int i = 0; i <= d; ++i) {
-                if (A.grad_dtype == NIS_F64) reinterpret_cast<double*>(A.grad_in)[pt * rowlen + i] = (double)g[i];
-                else reinterpret_cast<float*>(A.grad_in)[pt * rowlen + i] = g[i];
-            }
-        }
+        if (A.grad_in)
+            for (int i = 0; i <= d; ++i) store_io(A.grad_in, A.grad_dtype, pt * rowlen + i, g[i]);
     }
+}
+
+int launch_flow_bwd_tail(const DevFlow& F, const BwdTailArgs& A, cudaStream_t s) {
+    const long long blocks = (A.B + 255) / 256;
+    flow_bwd_tail_kernel<<<(int)(blocks < NIS_MAX_GRID ? blocks : NIS_MAX_GRID), 256, 0, s>>>(F, A);
+    NIS_CUDA_CHECK_LAUNCH();
+    return NIS_OK;
 }
 
 // grad_params[cell] += per-CTA slices (fixed order).  blockIdx.y = linear layer.
@@ -898,11 +883,8 @@ bool nis_tc_supported(const DevFlow& F) {
 
 bool nis_bwd_tc_supported(const DevFlow& F) { return F.kind == NIS_KIND_PWLIN && nis_tc_supported(F); }
 
-static int bt_grid(int64_t B) {
-    const int sms = nis_sm_count();
-    const long long npairs = ((B + TCM - 1) / TCM + 1) / 2;
-    return (int)(npairs < sms ? npairs : sms);
-}
+// CTAs of the head and layer launches at most (a B200's SM count): bt_carve reserves one wgrad slice per layer CTA
+#define BT_MAX_CTAS 148
 
 struct BtScratch { float *gstate, *zbuf, *dl, *dh[2], *bnb, *slices, *bdpack; size_t floats; };
 static void bt_carve(const DevFlow& F, int64_t B, float* base, BtScratch* s) {
@@ -915,7 +897,7 @@ static void bt_carve(const DevFlow& F, int64_t B, float* base, BtScratch* s) {
     s->dh[0] = base + off; off = up(off + tiles * BT_TILE);
     s->dh[1] = base + off; off = up(off + tiles * BT_TILE);
     s->bnb = base + off; off = up(off + (size_t)(F.depth + 1) * 2 * F.maxW);
-    s->slices = base + off; off = up(off + (size_t)(F.depth + 1) * 148 * 2 * 128 * TCH);
+    s->slices = base + off; off = up(off + (size_t)(F.depth + 1) * BT_MAX_CTAS * 2 * 128 * TCH);
     s->bdpack = base + off; off = up(off + (size_t)F.n_cells * bd_cell_floats(F));
     s->floats = off;
 }
@@ -926,35 +908,32 @@ size_t nis_bwd_tc_scratch_floats(const DevFlow& F, int64_t B) {
     return s.floats;
 }
 
-int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                         const float* saved, const float* bn_saved, const void* grad_out, int grad_dtype,
-                         float* grad_params, void* grad_in, int64_t B, cudaStream_t s) {
+int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* saved,
+                         const float* bn_saved, const void* grad_out, int grad_dtype, float* grad_params, void* grad_in,
+                         int64_t B, cudaStream_t s) {
     BtScratch sc;
     bt_carve(F, B, ws.bwd, &sc);
-    int grid = bt_grid(B);
-    if (grid > 148) grid = 148;
-    cudaMemsetAsync(ws.counter, 0, 256, s);
-    int rc = launch_flow_pack(F, params, bn_running, ws.wpack, NIS_BN_TRAIN, s);
-    if (rc) return rc;
-    flow_bwd_tc_pack_kernel<<<dim3(16, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.bdpack);
+    const long long ntiles = (B + TCM - 1) / TCM;
+    const int sms = nis_sm_count(), ctas = sms < BT_MAX_CTAS ? sms : BT_MAX_CTAS;
+    const int grid = (int)((ntiles + 1) / 2 < ctas ? (ntiles + 1) / 2 : ctas);    // head: two tiles at a time per CTA
+    const int lgrid = (int)(ntiles < ctas ? ntiles : ctas);                       // layers: one tile at a time, one slice each
+    flow_bwd_tc_pack_kernel<<<dim3(16, F.n_cells), 256, 0, s>>>(F, params, sc.bdpack);
     NIS_CUDA_CHECK_LAUNCH();
-    rc = nis_tc_pack(F, params, ws.tcpack, s);
+    int rc = nis_tc_pack(F, params, ws.tcpack, s);
     if (rc) return rc;
     BtArgs A;
-    A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype; A.grad_in = nullptr;
+    A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype;
     A.gstate = sc.gstate; A.params = params; A.wpack = ws.wpack; A.bn_saved = bn_saved;
     A.tcpack = ws.tcpack; A.bdpack = sc.bdpack; A.zbuf = sc.zbuf; A.dl = sc.dl;
     A.bnb = sc.bnb; A.slices = sc.slices; A.grad_params = grad_params;
-    A.partials = ws.partials; A.counter = ws.counter; A.B = B; A.ntiles = (B + TCM - 1) / TCM; A.grid = grid;
-    A.dh_in = nullptr; A.dh_out = nullptr; A.lam = 0; A.flush_every = BT_FLUSH;
+    A.partials = ws.partials; A.counter = ws.counter; A.B = B; A.ntiles = ntiles; A.grid = lgrid;
+    A.dh_in = nullptr; A.dh_out = nullptr; A.lam = 0;
+    BwdTailArgs Ta;
+    Ta.saved = saved; Ta.gstate = sc.gstate; Ta.wpack = ws.wpack; Ta.bn_saved = bn_saved; Ta.bnb = sc.bnb;
+    Ta.grad_dtype = grad_dtype; Ta.B = B; Ta.tile_floats = BT_TILE;
     const size_t smem64 = (size_t)bt_layout(64).total + 1024, smem128 = (size_t)bt_layout(128).total + 1024;
     NIS_ENSURE_SMEM((flow_bwd_tc_layer_kernel<64>), (int)smem64);
     NIS_ENSURE_SMEM((flow_bwd_tc_layer_kernel<128>), (int)smem128);
-    const int sms1 = nis_sm_count();
-    const long long nt1 = (B + TCM - 1) / TCM;
-    const int grid1 = (int)(nt1 < sms1 ? nt1 : sms1);
-    const int lgrid = grid1;                               // CTAs of the layer launches (one tile at a time each) = slices per layer
-    A.grid = lgrid;
     for (int c = F.n_cells - 1; c >= 0; --c) {
         A.c = c; A.first = c == F.n_cells - 1;
         const size_t smem_head = (size_t)tc_layout(F, F.cells[c].P, 1, F.depth, false).total + 2 * (F.d + 1) * TCM * 4 + 1024;
@@ -970,12 +949,9 @@ int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float*
             NIS_CUDA_CHECK_LAUNCH();
             pp ^= 1;
         }
-        A.dh_in = sc.dh[pp];
-        A.grad_in = c == 0 ? grad_in : nullptr;
-        long long blocks = (B + 255) / 256;
-        flow_bwd_tc_tail_kernel<<<(int)(blocks < 1184 ? blocks : 1184), 256, 0, s>>>(F, A);
-        NIS_CUDA_CHECK_LAUNCH();
-        A.grad_in = nullptr;
+        Ta.c = c; Ta.dh_in = sc.dh[pp]; Ta.grad_in = c == 0 ? grad_in : nullptr;
+        rc = launch_flow_bwd_tail(F, Ta, s);
+        if (rc) return rc;
         flow_bwd_tc_reduce_kernel<<<dim3(128, F.depth + 1), 256, 0, s>>>(F, sc.slices, lgrid, c, grad_params);
         NIS_CUDA_CHECK_LAUNCH();
     }

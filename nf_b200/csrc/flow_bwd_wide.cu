@@ -19,7 +19,8 @@
 //               MMAs; the accumulator lives in tensor memory and is flushed to the CTA's slice every 8 tiles (tcgen05
 //               accumulation truncates; the first flush stores, the later ones are vector reductions); a fixed-order
 //               reduce adds the slices.
-//   tail      : BatchNorm backward of the input normalisation (flow_bwd_tc.cu's kernel).
+//   tail      : BatchNorm backward of the input normalisation (flow_bwd_tail_kernel of flow_bwd_tc.cu, with this file's
+//               tile stride).
 #include <stdlib.h>
 #include "common.cuh"
 #include "spline.cuh"
@@ -60,9 +61,8 @@ __host__ __device__ static inline size_t bw_dg_cell_floats(const DevFlow& F) {
     return bw_dg_off(F, F.depth) + (size_t)F.widths[0] * bw_kout(F, bw_tmax(F)) * 2;
 }
 
-// W^T as K-panels of 32 upstream features: [N rows = input feature][32] hi then lo; + this batch's BN scale/shift
-__global__ void flow_bwd_wide_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_saved,
-                                          float* __restrict__ wpack, float* __restrict__ dgpack) {
+// W^T as K-panels of 32 upstream features: [N rows = input feature][32] hi then lo
+__global__ void flow_bwd_wide_pack_kernel(DevFlow F, const float* __restrict__ params, float* __restrict__ dgpack) {
     const int c = blockIdx.y;
     const DevCell& q = F.cells[c];
     const float* p = params + q.param_off;
@@ -94,21 +94,6 @@ __global__ void flow_bwd_wide_pack_kernel(DevFlow F, const float* __restrict__ p
             *reinterpret_cast<float*>(panel + (size_t)N * 128 + off) = tf32_rn(v - h);
         }
     }
-    for (int l = 0; l <= F.depth; ++l) {
-        const int Wl = F.W(c, l), Wp = F.Wp(c, l);
-        const long long g = F.p_bn_gamma(c, l);
-        const float* sv = bn_saved + q.sv_off + l * 2 * F.maxW;
-        float* aff = wpack + q.pk_off + q.aff_off[l];
-        for (int j = (int)tid; j < Wp; j += (int)nth) {
-            float sc = 0.f, sh = 0.f;
-            if (j < Wl) { sc = p[g + j] * sv[F.maxW + j]; sh = p[g + Wl + j] - sv[j] * sc; }
-            aff[j] = sc; aff[Wp + j] = sh;
-        }
-    }
-}
-
-__device__ __forceinline__ float bw_load_g(const void* p, int dtype, long long idx) {
-    return dtype == NIS_F64 ? (float)reinterpret_cast<const double*>(p)[idx] : reinterpret_cast<const float*>(p)[idx];
 }
 
 // ===================================================================================================
@@ -258,8 +243,8 @@ __global__ void __launch_bounds__(WD_THREADS, 1) flow_bwd_wide_head_kernel(const
                 for (int i = 0; i <= d; ++i) st[i * TCM] = sv[i];
                 Jout = A.saved[((long long)(c + 1) * A.B + pt) * rowlen + d];
                 if (A.first) {
-                    for (int i = 0; i < d; ++i) gr[F.out_perm[i] * TCM] = bw_load_g(A.grad_out, A.grad_dtype, pt * rowlen + i);
-                    gr[d * TCM] = bw_load_g(A.grad_out, A.grad_dtype, pt * rowlen + d);
+                    for (int i = 0; i < d; ++i) gr[F.out_perm[i] * TCM] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + i);
+                    gr[d * TCM] = load_io(A.grad_out, A.grad_dtype, pt * rowlen + d);
                 } else {
                     for (int i = 0; i <= d; ++i) gr[i * TCM] = A.gstate[pt * rowlen + i];
                 }
@@ -911,37 +896,6 @@ __global__ void flow_bwd_wide_reduce_kernel(DevFlow F, const float* __restrict__
     }
 }
 
-// tail of flow_bwd_tc.cu, reused with the wide tile stride
-struct BtTailArgs { const float* saved; float* gstate; const float* dh_in; const float* wpack; const float* bn_saved; const float* bnb;
-                    void* grad_in; int grad_dtype; long long B; int c, tile_floats; };
-__global__ void __launch_bounds__(256) flow_bwd_wide_tail_kernel(const __grid_constant__ DevFlow F, const BtTailArgs A) {
-    const int c = A.c;
-    const DevCell& q = F.cells[c];
-    const int d = F.d, maxW = F.maxW;
-    const long long rowlen = d + 1;
-    const float* pk = A.wpack + q.pk_off;
-    const float* sv = A.bn_saved + q.sv_off;
-    for (long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x; pt < A.B; pt += (long long)gridDim.x * blockDim.x) {
-        const float* xs = A.saved + ((long long)c * A.B + pt) * rowlen;
-        float* gs = A.gstate + pt * rowlen;
-        const float* da = A.dh_in + (size_t)(pt >> 7) * A.tile_floats + (pt & 127);
-        float g[NIS_MAX_DIM + 1];
-        for (int i = 0; i <= d; ++i) g[i] = gs[i];
-        for (int k = 0; k < q.P; ++k) {
-            const int col = q.feed[k];
-            const float xh = (xs[col] - sv[k]) * sv[maxW + k];
-            g[col] += pk[q.aff_off[0] + k] * (da[(size_t)k * TCM] - A.bnb[k] - xh * A.bnb[maxW + k]);
-        }
-        for (int i = 0; i <= d; ++i) gs[i] = g[i];
-        if (A.grad_in) {
-            for (int i = 0; i <= d; ++i) {
-                if (A.grad_dtype == NIS_F64) reinterpret_cast<double*>(A.grad_in)[pt * rowlen + i] = (double)g[i];
-                else reinterpret_cast<float*>(A.grad_in)[pt * rowlen + i] = g[i];
-            }
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------
 bool nis_bwd_wide_supported(const DevFlow& F) {
     if (!nis_wide_supported(F, NIS_BN_TRAIN)) return false;
@@ -954,6 +908,9 @@ bool nis_bwd_wide_supported(const DevFlow& F) {
     if (bw_dg_layout(F, 1).slots < 2) return false;
     return true;
 }
+
+// wgrad slices: one [128][128] accumulator per CTA of a wgrad launch (row block x column block x part of the tiles)
+#define BW_SLICES 320
 
 struct BwScratch { float *gstate, *zbuf, *dl, *dh[2], *dz, *bnb, *slices, *dgpack; size_t floats; };
 static void bw_carve(const DevFlow& F, int64_t B, float* base, BwScratch* s) {
@@ -968,7 +925,7 @@ static void bw_carve(const DevFlow& F, int64_t B, float* base, BwScratch* s) {
     s->dh[1] = base + off; off = up(off + tiles * W * TCM);
     s->dz = base + off; off = up(off + tiles * W * TCM);
     s->bnb = base + off; off = up(off + (size_t)(F.depth + 1) * 2 * F.maxW);
-    s->slices = base + off; off = up(off + (size_t)320 * 128 * 128);
+    s->slices = base + off; off = up(off + (size_t)BW_SLICES * 128 * 128);
     s->dgpack = base + off; off = up(off + (size_t)F.n_cells * bw_dg_cell_floats(F));
     s->floats = off;
 }
@@ -978,8 +935,8 @@ size_t nis_bwd_wide_scratch_floats(const DevFlow& F, int64_t B) {
     return s.floats;
 }
 
-int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                           const float* saved, const float* bn_saved, const float* act_saved, const void* grad_out, int grad_dtype,
+int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* saved,
+                           const float* bn_saved, const float* act_saved, const void* grad_out, int grad_dtype,
                            float* grad_params, void* grad_in, int64_t B, cudaStream_t s) {
     BwScratch sc;
     bw_carve(F, B, ws.bwd, &sc);
@@ -987,12 +944,9 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
     const long long ntiles = (B + TCM - 1) / TCM;
     const int grid = (int)(ntiles < sms ? ntiles : sms);
     const int W = F.widths[0], Kp = wd_kp16(F), depth = F.depth;
-    cudaMemsetAsync(ws.counter, 0, 256, s);
-    int rc = launch_flow_pack(F, params, bn_running, ws.wpack, NIS_BN_TRAIN, s);
-    if (rc) return rc;
-    flow_bwd_wide_pack_kernel<<<dim3(128, F.n_cells), 256, 0, s>>>(F, params, bn_saved, ws.wpack, sc.dgpack);
+    flow_bwd_wide_pack_kernel<<<dim3(128, F.n_cells), 256, 0, s>>>(F, params, sc.dgpack);
     NIS_CUDA_CHECK_LAUNCH();
-    rc = nis_wide_pack(F, params, ws.tcpack, s);
+    int rc = nis_wide_pack(F, params, ws.tcpack, s);
     if (rc) return rc;
     BwArgs A;
     A.saved = saved; A.grad_out = grad_out; A.grad_dtype = grad_dtype; A.gstate = sc.gstate;
@@ -1001,6 +955,9 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
     A.partials = ws.partials; A.counter = ws.counter; A.B = B; A.ntiles = ntiles;
     A.dh_in = nullptr; A.dh_out = nullptr; A.lam = 0; A.nparts = 1;
     const size_t tile_fl = (size_t)W * TCM;
+    BwdTailArgs Ta;
+    Ta.saved = saved; Ta.gstate = sc.gstate; Ta.wpack = ws.wpack; Ta.bn_saved = bn_saved; Ta.bnb = sc.bnb;
+    Ta.grad_dtype = grad_dtype; Ta.B = B; Ta.tile_floats = (int)tile_fl;
     const long long rows = (long long)B * (F.d + 1);
     auto headk = F.kind == NIS_KIND_PWLIN ? flow_bwd_wide_head_kernel<NIS_KIND_PWLIN> : flow_bwd_wide_head_kernel<NIS_KIND_PWQUAD>;
     NIS_ENSURE_SMEM((flow_bwd_wide_wgrad_kernel<true>), 196608 + 1024);
@@ -1055,7 +1012,7 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
             const int nrb = (nrows + 63) / 64, nnh = lam == 0 ? 1 : (W + 127) / 128;
             int nparts = (2 * sms) / (nrb * nnh);
             if (nparts < 1) nparts = 1;
-            if (nparts > 320 / (nrb * nnh)) nparts = 320 / (nrb * nnh);
+            if (nparts > BW_SLICES / (nrb * nnh)) nparts = BW_SLICES / (nrb * nnh);
             if (nparts > ntiles) nparts = (int)ntiles;
             if (nparts < 1) return NIS_EUNSUPPORTED;
             A.nparts = nparts;
@@ -1067,12 +1024,9 @@ int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const floa
             NIS_CUDA_CHECK_LAUNCH();
         }
         // ---- tail ------------------------------------------------------------------------------------------------------
-        BtTailArgs Ta;
-        Ta.saved = saved; Ta.gstate = sc.gstate; Ta.dh_in = sc.dh[pp]; Ta.wpack = ws.wpack; Ta.bn_saved = bn_saved; Ta.bnb = sc.bnb;
-        Ta.grad_in = c == 0 ? grad_in : nullptr; Ta.grad_dtype = grad_dtype; Ta.B = B; Ta.c = c; Ta.tile_floats = (int)tile_fl;
-        long long blocks = (B + 255) / 256;
-        flow_bwd_wide_tail_kernel<<<(int)(blocks < 1184 ? blocks : 1184), 256, 0, s>>>(F, Ta);
-        NIS_CUDA_CHECK_LAUNCH();
+        Ta.c = c; Ta.dh_in = sc.dh[pp]; Ta.grad_in = c == 0 ? grad_in : nullptr;
+        rc = launch_flow_bwd_tail(F, Ta, s);
+        if (rc) return rc;
     }
     return NIS_OK;
 }

@@ -19,26 +19,32 @@
 #include "flow_host.cuh"
 
 // ---------------------------------------------------------------------------------------------------
-// repack: torch-layout params -> transposed zero-padded weights (+ eval-mode BN scale/shift)
+// repack: torch-layout params -> transposed zero-padded weights (+ BN scale/shift: eval mode from the running statistics;
+// train mode from bn_saved, the batch statistics a forward saved, for its backward; none in a train-mode forward, whose
+// statistics passes write them)
 // grid = (blocks, n_cells)
 // ---------------------------------------------------------------------------------------------------
 __global__ void flow_pack_kernel(DevFlow F, const float* __restrict__ params, const float* __restrict__ bn_running,
-                                 float* __restrict__ wpack, int bn_mode) {
+                                 const float* __restrict__ bn_saved, float* __restrict__ wpack, int bn_mode) {
     const int c = blockIdx.y;
     const DevCell& q = F.cells[c];
     const float* p = params + q.param_off;
     float* pk = wpack + q.pk_off;
     const int tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
-    if (bn_mode == NIS_BN_EVAL) {
-        const float* rs = bn_running + q.bn_off;
+    if (bn_mode == NIS_BN_EVAL || bn_saved) {
         for (int l = 0; l <= F.depth; ++l) {
             const int W = F.W(c, l), Wp = F.Wp(c, l);
             const long long g = F.p_bn_gamma(c, l), r = F.r_mean(c, l);
             for (int j = tid; j < Wp; j += nth) {
                 float sc = 0.f, sh = 0.f;
-                if (j < W) {
+                if (j < W && bn_mode == NIS_BN_EVAL) {
+                    const float* rs = bn_running + q.bn_off;
                     sc = p[g + j] / sqrtf(rs[r + W + j] + F.eps);
                     sh = p[g + W + j] - rs[r + j] * sc;
+                } else if (j < W) {
+                    const float* sv = bn_saved + q.sv_off + l * 2 * F.maxW;
+                    sc = p[g + j] * sv[F.maxW + j];
+                    sh = p[g + W + j] - sv[j] * sc;
                 }
                 pk[q.aff_off[l] + j] = sc;
                 pk[q.aff_off[l] + Wp + j] = sh;
@@ -80,8 +86,9 @@ int nis_pack_blocks(const DevFlow& F) {
     return bx > 64 ? 64 : bx;
 }
 
-int launch_flow_pack(const DevFlow& F, const float* params, const float* bn_running, float* wpack, int bn_mode, cudaStream_t s) {
-    flow_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, bn_running, wpack, bn_mode);
+int launch_flow_pack(const DevFlow& F, const float* params, const float* bn_running, const float* bn_saved, float* wpack,
+                     int bn_mode, cudaStream_t s) {
+    flow_pack_kernel<<<dim3(nis_pack_blocks(F), F.n_cells), 256, 0, s>>>(F, params, bn_running, bn_saved, wpack, bn_mode);
     NIS_CUDA_CHECK_LAUNCH();
     return NIS_OK;
 }
@@ -525,7 +532,7 @@ static int fwd_prologue(const NisFlowDesc* desc, const float* params, const floa
     nis_flow_carve(F, B, workspace, &ws);
     cudaMemsetAsync(ws.counter, 0, 256, s);
     timing_mark(s, -1);                     // open the first interval on this stream (after the counter memset)
-    rc = launch_flow_pack(F, params, bn_running, ws.wpack, bn_mode, s);
+    rc = launch_flow_pack(F, params, bn_running, nullptr, ws.wpack, bn_mode, s);   // bn_saved: filled by this forward
     if (rc) return rc;
     timing_mark(s, 0);
     A.in = in; A.in_dtype = in_dtype; A.in_cols = in_cols;

@@ -32,14 +32,6 @@ struct FwdArgs {
 static_assert(std::is_trivially_copyable<FwdArgs>::value, "FwdArgs is a kernel argument");
 
 
-__device__ __forceinline__ float load_io(const void* p, int dtype, long long idx) {
-    return dtype == NIS_F64 ? (float)reinterpret_cast<const double*>(p)[idx] : reinterpret_cast<const float*>(p)[idx];
-}
-__device__ __forceinline__ void store_io(void* p, int dtype, long long idx, float v) {
-    if (dtype == NIS_F64) reinterpret_cast<double*>(p)[idx] = (double)v; else reinterpret_cast<float*>(p)[idx] = v;
-}
-
-
 // Train-mode BN statistics: every CTA of a statistics pass hands in its float64 per-feature sums
 // (sacc[0..maxW) = sum z, sacc[maxW..2maxW) = sum z^2, in shared memory); the last CTA to arrive adds
 // the per-CTA partials in index order (deterministic) and folds them into the layer's scale/shift

@@ -23,9 +23,11 @@ bool nis_tiled_supported(const DevFlow& F);               // flow_tiled.cu
 bool nis_moments_supported(const DevFlow& F, int c);      // flow_tiled.cu
 
 // ---- flow_fwd.cu -------------------------------------------------------------------------------------------------------
-// torch-layout parameters -> wpack (flow_pack_kernel), and the x-extent of its grid (y: one row of blocks per cell)
+// torch-layout parameters -> wpack (flow_pack_kernel), and the x-extent of its grid (y: one row of blocks per cell).
+// BN scale/shift: eval mode from bn_running; train mode from bn_saved, or none when bn_saved is null.
 int nis_pack_blocks(const DevFlow& F);
-int launch_flow_pack(const DevFlow& F, const float* params, const float* bn_running, float* wpack, int bn_mode, cudaStream_t s);
+int launch_flow_pack(const DevFlow& F, const float* params, const float* bn_running, const float* bn_saved, float* wpack,
+                     int bn_mode, cudaStream_t s);
 
 // ---- workspace: pack and scratch sizes ---------------------------------------------------------------------------------
 size_t nis_tc_pack_floats(const DevFlow& F);              // flow_bwd_tc.cu
@@ -44,10 +46,18 @@ int nis_launch_tiled(const DevFlow& F, const FwdArgs& A, cudaStream_t s);       
 int nis_launch_col_stats(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
 int nis_launch_col_moments(const DevFlow& F, const FwdArgs& A, cudaStream_t s);
 
-// ---- train-mode backwards ----------------------------------------------------------------------------------------------
-int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                         const float* saved, const float* bn_saved, const void* grad_out, int grad_dtype,
-                         float* grad_params, void* grad_in, int64_t B, cudaStream_t s);                   // flow_bwd_tc.cu
-int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* bn_running,
-                           const float* saved, const float* bn_saved, const float* act_saved, const void* grad_out,
-                           int grad_dtype, float* grad_params, void* grad_in, int64_t B, cudaStream_t s); // flow_bwd_wide.cu
+// ---- train-mode backwards: launches after nis_flow_backward_cached's counter memset and flow_pack_kernel ---------------
+int nis_flow_backward_tc(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* saved,
+                         const float* bn_saved, const void* grad_out, int grad_dtype, float* grad_params, void* grad_in,
+                         int64_t B, cudaStream_t s);                                                       // flow_bwd_tc.cu
+int nis_flow_backward_wide(const DevFlow& F, const FlowWorkspace& ws, const float* params, const float* saved,
+                           const float* bn_saved, const float* act_saved, const void* grad_out, int grad_dtype,
+                           float* grad_params, void* grad_in, int64_t B, cudaStream_t s);                  // flow_bwd_wide.cu
+
+// BatchNorm backward of a cell's input normalisation, dL/dx of its pass-through columns (flow_bwd_tc.cu): the last launch of
+// a cell in both tensor-core backwards.  dh_in holds dL/dh_0 in 128-point tiles of tile_floats floats.
+struct BwdTailArgs {
+    const float* saved; float* gstate; const float* dh_in; const float* wpack; const float* bn_saved; const float* bnb;
+    void* grad_in; int grad_dtype; long long B; int c, tile_floats;
+};
+int launch_flow_bwd_tail(const DevFlow& F, const BwdTailArgs& A, cudaStream_t s);

@@ -31,10 +31,10 @@ WIDE_EVAL = ("flow_wide_pack_kernel", "flow_wide_tc_kernel") + PACK
 TILED_FWD = ("flow_cell_tiled_kernel", "flow_col_moments_kernel") + PACK
 GENERIC = ("flow_fwd_generic_kernel",) + PACK
 COOP = ("flow_fwd_coop_kernel",) + PACK
-BWD_TC = ("flow_bwd_tc_head_kernel", "flow_bwd_tc_layer_kernel", "flow_bwd_tc_pack_kernel", "flow_bwd_tc_reduce_kernel",
-          "flow_bwd_tc_tail_kernel", "flow_tc_pack_kernel") + PACK
-BWD_WIDE_CACHED = ("flow_bwd_wide_dgrad_kernel", "flow_bwd_wide_head_kernel", "flow_bwd_wide_pack_kernel",
-                   "flow_bwd_wide_reduce_kernel", "flow_bwd_wide_tail_kernel", "flow_bwd_wide_wgrad_kernel",
+BWD_TC = ("flow_bwd_tail_kernel", "flow_bwd_tc_head_kernel", "flow_bwd_tc_layer_kernel", "flow_bwd_tc_pack_kernel",
+          "flow_bwd_tc_reduce_kernel", "flow_tc_pack_kernel") + PACK
+BWD_WIDE_CACHED = ("flow_bwd_tail_kernel", "flow_bwd_wide_dgrad_kernel", "flow_bwd_wide_head_kernel",
+                   "flow_bwd_wide_pack_kernel", "flow_bwd_wide_reduce_kernel", "flow_bwd_wide_wgrad_kernel",
                    "flow_wide_pack_kernel") + PACK
 BWD_WIDE = BWD_WIDE_CACHED + ("flow_wide_tc_kernel",)            # layer passes run again: no activation cache
 BWD_GENERIC = ("bwd_reduce_gpart_kernel", "flow_bwd_generic_kernel", "flow_bwd_pack_kernel") + PACK
